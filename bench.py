@@ -3,7 +3,7 @@
 4096 stereo float streams, 44.1 -> 48 kHz, 256-tap ART filters (256 phases, Blackman-Harris,
 inter-phase interpolation), 1 s of audio per stream per step, on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  `value` = whole-job output Msamples/s with inputs
 resident in HBM; `e2e` = the same through the host-buffer C-ABI call (pinned host
@@ -23,6 +23,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the tree may be read-only: leave no __pycache__ in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "tests")):
     if p not in sys.path:
@@ -552,6 +553,26 @@ def bench_c5(espb, ranks, stream, peak_tf, link, steps, want_e2e, checks):
     return rec
 
 
+DUMP_STREAMS = 64  # 64 streams x 95726 output samples x 4 bytes = 24.5 MB per dump
+
+
+def dump_outputs(espb, path, d_out, out_row, ns, used, gen, stream):
+    """What a caller of the timed path holds after its last step: the frame counts and the output of a fixed, seeded
+    sample of this rank's streams, as .npy files (float32 samples, float64 counts and stream indices), so that two
+    builds can be compared output for output on the same inputs."""
+    L = espb.lib()
+    rows = np.sort(np.random.default_rng(0).choice(ns, size=min(ns, DUMP_STREAMS), replace=False))
+    y = np.empty((rows.size, gen * CHANNELS), f32)
+    for k, r in enumerate(rows):
+        espb.capi._check(L.espb_memcpy_d2h(y[k].ctypes.data, d_out.ptr + int(r) * out_row * 4, y[k].nbytes, stream),
+                         "d2h")
+    espb.capi._check(L.espb_stream_sync(stream), "sync")
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "output.npy"), y)
+    np.save(os.path.join(path, "output_streams.npy"), rows.astype(np.float64))
+    np.save(os.path.join(path, "frames_used_generated.npy"), np.array([used, gen], np.float64))
+
+
 def run_checks(checks, mode):
     """CPU leg (rank 0, N = 1): one stream of every sub-record re-computed by the CPU restatement of the reference."""
     from oracle_lib import Oracle
@@ -614,6 +635,8 @@ def main():
     ap.add_argument("--configs", default="C5,C3,C4", help="which sub-records to run (comma-separated)")
     ap.add_argument("--mode", default="fast", choices=["fast", "exact"],
                     help="arithmetic of the dot products: fast = FFMA2 chain (the metric), exact = un-fused, bit-exact")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (a fixed sample of its streams) as DIR/*.npy")
     args = ap.parse_args()
     out = protect_stdout()
     if args.impl == "reference":
@@ -688,6 +711,8 @@ def main():
     used, gen = st["r"]
     launches = espb.launch_count() - launches0
     total_ms = ranks.max(float(ms.value))  # device-timed, max over ranks (gathered by ncclAllGather)
+    if args.dump_outputs and rank == 0:  # before the second loop below overwrites d_out
+        dump_outputs(espb, args.dump_outputs, d_out, out_row, ns, used, gen, stream)
 
     # ---- second timed loop, same steps, with CUDA events around every launch of the resampler kernel (the roofline's
     # numerator).  In the loop above the kernel starts while the staging kernel is still running (programmatic

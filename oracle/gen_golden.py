@@ -4,10 +4,12 @@ Run in the build container (needs oracle/_ref, i.e. /root/reference present):
     python oracle/gen_golden.py
 Every array written here is an output of the real reference library
 (oracle/_ref/libesp_audio_ref.so, built by oracle/Makefile from /root/reference),
-never of the oracle port or of the CUDA path.  Inputs are stored next to the
-outputs for the small cases; the large cases store SHA-256 digests, frame counts
-and final state, with inputs regenerated from the seeded generators in
-tests/oracle_lib.py (an input digest guards against generator drift).
+never of the oracle port or of the CUDA path.  Inputs drawn from the seeded
+generators in tests/signals.py are stored as their recipe and SHA-256 digest
+(meta "inputs"; tests/conftest.py regenerates them), other inputs next to the
+outputs; the large cases store SHA-256 digests, frame counts and final state,
+with inputs regenerated from the same generators (an input digest guards
+against generator drift).
 """
 import hashlib
 import json
@@ -18,8 +20,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
-from oracle_lib import (BLACKMAN_HARRIS, INCLUDE_LOWPASS, SUBSAMPLE_INTERPOLATE, Reference, multitone,  # noqa: E402
-                        noise)
+from oracle_lib import BLACKMAN_HARRIS, INCLUDE_LOWPASS, SUBSAMPLE_INTERPOLATE, Reference, noise  # noqa: E402
+from signals import from_recipe  # noqa: E402
 
 R = Reference()
 OUT = os.path.join(ROOT, "tests", "golden")
@@ -31,7 +33,14 @@ def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
-arrays, meta = {}, {}
+arrays, meta = {}, {"inputs": {}}
+
+
+def seeded_input(name, **recipe):
+    """A signal of tests/signals.py: stored as its recipe and digest (tests/conftest.py regenerates it), not as data."""
+    x = from_recipe(recipe)
+    meta["inputs"][name] = dict(recipe, sha256=sha(x))
+    return x
 
 # ---- 1. filter banks ---------------------------------------------------------
 BANKS = [  # taps, filters, lowpass, flags
@@ -71,14 +80,16 @@ SMALL = [  # name, channels, taps, filters, lowpass, flags, ratio, n_in, advance
 ]
 meta["small"] = []
 for name, ch, taps, filters, lp, flags, ratio, n_in, adv, sig in SMALL:
-    x = multitone(n_in, ch, 44100.0, stream=5, amp=0.9) if sig == "multitone" else noise(n_in, ch, stream=11, amp=0.9)
+    if sig == "multitone":
+        x = seeded_input(f"small_{name}_x", signal=sig, frames=n_in, channels=ch, stream=5, amp=0.9, fs=44100.0)
+    else:
+        x = seeded_input(f"small_{name}_x", signal=sig, frames=n_in, channels=ch, stream=11, amp=0.9)
     ctx = R.resampler(ch, taps, filters, lp, flags)
     if adv:
         ctx.advance(adv)
     cap = int(n_in * float(ratio)) + 64
     y, used, gen = ctx.process_interleaved(x, cap, ratio)
     off, idx = ctx.state()
-    arrays[f"small_{name}_x"] = x
     arrays[f"small_{name}_y"] = y
     meta["small"].append(dict(name=name, channels=ch, taps=taps, filters=filters, lowpass=lp, flags=flags,
                               ratio=float(ratio), n_in=n_in, advance=adv, cap=cap, used=used, generated=gen,
@@ -87,7 +98,7 @@ for name, ch, taps, filters, lp, flags, ratio, n_in, adv, sig in SMALL:
 # chunked == one-shot (KAT 7) and output-capacity-limited calls: store the chunk plan + per-call results
 rng = np.random.default_rng(2024)
 ch, taps, filters, ratio = 2, 64, 64, f32(48000) / f32(44100)
-x = noise(6000, ch, stream=2, amp=0.8)
+x = seeded_input("chunked_x", signal="noise", frames=6000, channels=ch, stream=2, amp=0.8)
 ctx = R.resampler(ch, taps, filters, 1.0, 3)
 ctx.advance(taps / 2)
 plan, outs, pos = [], [], 0
@@ -98,7 +109,6 @@ while pos < 6000:
     plan.append((n_in, n_out, used, gen))
     outs.append(y)
     pos += used
-arrays["chunked_x"] = x
 arrays["chunked_plan"] = np.array(plan, np.int64)
 arrays["chunked_y"] = np.concatenate(outs)
 meta["chunked"] = dict(channels=ch, taps=taps, filters=filters, ratio=float(ratio), flags=3, advance=taps / 2)
@@ -157,8 +167,7 @@ meta["kat"]["q2f32_quirk"] = float(R.quantized_to_float(np.array([0, 0, 0x80, 1]
 
 # ---- 5. biquad --------------------------------------------------------------------
 meta["biquad"] = []
-x = noise(4000, 2, stream=9, amp=0.9)
-arrays["biquad_x"] = x
+x = seeded_input("biquad_x", signal="noise", frames=4000, channels=2, stream=9, amp=0.9)
 for k, (kind, f, gain) in enumerate([("lp", 0.2274, 1.0), ("lp", 1.0 / 6.0, 1.0), ("lp", 0.441, 0.5),
                                      ("lp", 0.02, 1.0), ("hp", 0.1, 1.0), ("hp", 0.3, 2.0)]):
     c = R.biquad_lowpass(f) if kind == "lp" else R.biquad_highpass(f)

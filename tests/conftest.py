@@ -1,3 +1,4 @@
+import hashlib
 import json
 import os
 import sys
@@ -16,11 +17,26 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a real B200 (run with -m gpu on the GPU box)")
 
 
+class GoldenArrays(dict):
+    """Every access returns a fresh array, as np.load's NpzFile does: a test that writes into one cannot change what
+    the next test reads."""
+
+    def __getitem__(self, name):
+        return dict.__getitem__(self, name).copy()
+
+
 @pytest.fixture(scope="session")
 def golden():
-    arrays = np.load(os.path.join(HERE, "golden", "golden_v1.npz"))
+    """Stored arrays plus the seeded inputs, regenerated from their recipes and checked against their digests."""
+    from signals import from_recipe
+    with np.load(os.path.join(HERE, "golden", "golden_v1.npz")) as npz:
+        arrays = GoldenArrays({name: npz[name] for name in npz.files})
     with open(os.path.join(HERE, "golden", "golden_v1.json")) as fh:
         meta = json.load(fh)
+    for name, recipe in meta["inputs"].items():
+        x = from_recipe(recipe)
+        assert hashlib.sha256(x.tobytes()).hexdigest() == recipe["sha256"], f"{name}: tests/signals.py has drifted"
+        arrays[name] = x
     return arrays, meta
 
 
@@ -28,14 +44,6 @@ def golden():
 def oracle():
     from oracle_lib import Oracle
     return Oracle()
-
-
-@pytest.fixture(scope="session")
-def reference():
-    from oracle_lib import Reference, have_reference
-    if not have_reference():
-        pytest.skip("oracle/_ref not built (no /root/reference on this box)")
-    return Reference()
 
 
 def bits_equal(a, b):

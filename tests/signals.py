@@ -17,3 +17,10 @@ def noise(n_frames, channels, stream=0, amp=0.5):
     """uniform in [-A, A], seeded by 0xC0FFEE ^ stream, float32 interleaved."""
     rng = np.random.default_rng(0xC0FFEE ^ (stream * 7919 + 1))
     return ((rng.random(n_frames * channels) * 2.0 - 1.0) * amp).astype(np.float32)
+
+
+def from_recipe(r):
+    """The signal a recipe names: {"signal": "multitone" | "noise", "frames", "channels", "stream", "amp"[, "fs"]}."""
+    if r["signal"] == "multitone":
+        return multitone(r["frames"], r["channels"], r["fs"], stream=r["stream"], amp=r["amp"])
+    return noise(r["frames"], r["channels"], stream=r["stream"], amp=r["amp"])

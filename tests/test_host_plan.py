@@ -5,6 +5,9 @@ additionally proven by replaying it in numpy with the kernel's arithmetic (one
 accumulator per dot product, taps in order, FMUL+FADD) against the golden outputs."""
 import hashlib
 import os
+import subprocess
+import sys
+import textwrap
 
 import numpy as np
 import pytest
@@ -12,6 +15,7 @@ from conftest import bits_equal
 
 import esp_audio_libs_b200 as espb
 
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 f32 = np.float32
 
 
@@ -30,14 +34,23 @@ def test_library_loads_and_exports_every_declared_symbol():
 
 
 def test_no_cpu_fallback_fails_loudly():
-    if espb.device_count() > 0:
-        pytest.skip("a GPU is present")
-    with pytest.raises(espb.EspbError, match="no CUDA device"):
-        espb.ResampleBatch(2, 2, 64, 64, 1.0, 3)
-    with pytest.raises(espb.EspbError):
-        espb.BiquadBatch(4, 2, espb.biquad_lowpass(0.2))
-    with pytest.raises(espb.EspbError):
-        espb.Resampler(2, 1024, 4096, 44100, 48000, 16, 16, 2)
+    """Run in a child process with every CUDA device hidden, so that a machine with a GPU checks it too."""
+    code = textwrap.dedent(f"""
+        import sys
+        sys.path.insert(0, {ROOT!r})
+        import pytest
+        import esp_audio_libs_b200 as espb
+        assert espb.device_count() == 0
+        with pytest.raises(espb.EspbError, match="no CUDA device"):
+            espb.ResampleBatch(2, 2, 64, 64, 1.0, 3)
+        with pytest.raises(espb.EspbError):
+            espb.BiquadBatch(4, 2, espb.biquad_lowpass(0.2))
+        with pytest.raises(espb.EspbError):
+            espb.Resampler(2, 1024, 4096, 44100, 48000, 16, 16, 2)
+    """)
+    p = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=120)
+    assert p.returncode == 0, p.stderr[-2000:]
 
 
 def test_invalid_init_parameters():
