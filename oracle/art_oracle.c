@@ -2,8 +2,9 @@
  *
  * Plain-C restatement of the reference algorithm; every function names the
  * reference lines it follows (paths relative to /root/reference).  Arithmetic is
- * FP32, un-fused, in the reference's evaluation order.  Compile with
- * -ffp-contract=off.  Never linked into the product.
+ * FP32, un-fused, in the reference's evaluation order, except for the opt-in fmaf
+ * chain of orc_resample_set_fused.  Compile with -ffp-contract=off.  Never linked
+ * into the product.
  */
 #define _GNU_SOURCE
 #include "art_oracle.h"
@@ -25,16 +26,22 @@
 
 struct OrcResampler {
   int channels, ring_len, n_filters, taps, input_index, flags; /* include/art_resampler.h:25-29 */
+  int fused; /* not in the reference: orc_resample_set_fused */
   float output_offset;
   float *ring; /* channels x ring_len history (reference: buffers[ch]) */
   float *bank; /* (n_filters+1) x taps (reference: filters[i])       */
 };
 
-/* src/dsp/dsps_dotprod_f32_ansi.c:17-25 — sequential, separate multiply and add */
-static float orc_dot(const float *a, const float *b, int n) {
+/* src/dsp/dsps_dotprod_f32_ansi.c:17-25 — sequential, separate multiply and add.  With `fused` set, the same
+ * sequence with each multiply-add rounded once (correctly rounded fmaf): the library's fast mode (DESIGN.md §2.2). */
+static float orc_dot(const float *a, const float *b, int n, int fused) {
   float acc = 0;
-  for (int i = 0; i < n; i++)
-    acc += a[i] * b[i];
+  if (fused)
+    for (int i = 0; i < n; i++)
+      acc = fmaf(a[i], b[i], acc);
+  else
+    for (int i = 0; i < n; i++)
+      acc += a[i] * b[i];
   return acc;
 }
 
@@ -149,15 +156,16 @@ static float orc_subsample(const OrcResampler *r, const float *hist, float offse
     return *src;
   const float *win = src - taps / 2 + 1;
   if (!(r->flags & ORC_SUBSAMPLE_INTERPOLATE)) /* :428 nearest phase (may equal n_filters) */
-    return orc_dot(r->bank + (size_t) ((int) floorf(offset * (float) r->n_filters + 0.5f)) * taps, win, taps);
+    return orc_dot(r->bank + (size_t) ((int) floorf(offset * (float) r->n_filters + 0.5f)) * taps, win, taps,
+                   r->fused);
 
   offset *= (float) r->n_filters; /* :442 */
   int i = (int) floorf(offset);
-  float sum1 = orc_dot(r->bank + (size_t) i * taps, win, taps); /* :443 */
+  float sum1 = orc_dot(r->bank + (size_t) i * taps, win, taps, r->fused); /* :443 */
   offset -= (float) i;
   if (offset == 0.0f && !lowpass) /* :445 */
     return sum1;
-  float sum2 = orc_dot(r->bank + (size_t) (i + 1) * taps, win, taps); /* :448 */
+  float sum2 = orc_dot(r->bank + (size_t) (i + 1) * taps, win, taps, r->fused); /* :448 */
   return sum2 * offset + sum1 * (1.0f - offset);                       /* :450 */
 }
 
@@ -263,6 +271,7 @@ unsigned orc_resample_expected(const OrcResampler *r, int n_in, float ratio) {
 }
 
 int orc_resample_flags(const OrcResampler *r) { return r->flags; }
+void orc_resample_set_fused(OrcResampler *r, int fused) { r->fused = fused != 0; }
 void orc_resample_copy_filter(const OrcResampler *r, int idx, float *dst) {
   memcpy(dst, r->bank + (size_t) idx * r->taps, r->taps * sizeof(float));
 }
@@ -656,6 +665,11 @@ void orc_wrapper_free(OrcWrapper *w) {
   free(w->fin);
   free(w->fout);
   free(w);
+}
+
+void orc_wrapper_set_fused(OrcWrapper *w, int fused) {
+  if (w->art)
+    orc_resample_set_fused(w->art, fused);
 }
 
 int orc_wrapper_policy(const OrcWrapper *w, float coeffs[5], float *sample_ratio, float *art_lowpass,

@@ -13,7 +13,8 @@
  * the committed fixtures under tests/golden/ (made by oracle/gen_golden.py from
  * oracle/_ref) everywhere else.
  *
- * Must be compiled with -ffp-contract=off (the reference arithmetic is un-fused).
+ * Must be compiled with -ffp-contract=off (the reference arithmetic is un-fused; the one fused form,
+ * orc_resample_set_fused, calls fmaf explicitly).
  */
 #ifndef ART_ORACLE_H_
 #define ART_ORACLE_H_
@@ -48,6 +49,9 @@ void orc_resample_planar(OrcResampler *r, const float *const *in, int n_in, floa
 int orc_resample_flags(const OrcResampler *r);
 void orc_resample_copy_filter(const OrcResampler *r, int idx, float *dst);
 void orc_resample_state(const OrcResampler *r, float *output_offset, int *input_index);
+/* Not in the reference.  Non-zero: every dot product is an fmaf chain in tap order (one rounding per multiply-add),
+ * the library's fast mode (DESIGN.md §2.2); everything else is unchanged.  Per context, off by default. */
+void orc_resample_set_fused(OrcResampler *r, int fused);
 
 /* include/art_biquad.h:19-36 */
 typedef struct {
@@ -101,6 +105,8 @@ void orc_wrapper_resample(OrcWrapper *w, const uint8_t *in, uint8_t *out, size_t
                           float gain_db, uint64_t results[4]);
 /* policy introspection: pre(1)/post(2)/none(0), biquad coeffs, ART lowpass + flags */
 int orc_wrapper_policy(const OrcWrapper *w, float coeffs[5], float *sample_ratio, float *art_lowpass, int *art_flags);
+/* orc_resample_set_fused on the wrapper's resampler (no-op when the rates are equal) */
+void orc_wrapper_set_fused(OrcWrapper *w, int fused);
 
 /* CPU-baseline driver (bench.py cpu_baseline kind "port"): n_streams independent
  * contexts over n_threads host threads, processing time only, seconds. */

@@ -49,9 +49,17 @@ class _Backend:
     name = "?"
 
     # ---- ART resampler ----
-    def resampler(self, channels, taps, filters, lowpass, flags):
+    def resampler(self, channels, taps, filters, lowpass, flags, fused=False):
+        """fused=True: every dot product is an fmaf chain in tap order, the library's fast mode (oracle only)."""
+        self._check_fused(fused)
         h = self.f["init"](channels, taps, filters, lowpass, flags)
+        if h and fused:
+            self.lib.orc_resample_set_fused(h, 1)
         return ArtContext(self, h, channels, taps, filters) if h else None
+
+    def _check_fused(self, fused):
+        if fused:
+            raise ValueError(f"{self.name}: fused=True needs the oracle (the reference has no fused form)")
 
     # ---- quantisers ----
     def quantized_to_float(self, data, n, bits, gain_db=0.0):
@@ -83,9 +91,13 @@ class _Backend:
 
     # ---- wrapper ----
     def wrapper(self, in_samples, out_samples, src_rate, dst_rate, src_bits, dst_bits, channels, use_filter=True,
-                interpolate=True, taps=256, filters=256):
+                interpolate=True, taps=256, filters=256, fused=False):
+        """fused=True: the wrapper's resampler runs the fmaf chain (see resampler())."""
+        self._check_fused(fused)
         h = self.f["w_create"](in_samples, out_samples, src_rate, dst_rate, src_bits, dst_bits, channels,
                                int(use_filter), int(interpolate), taps, filters)
+        if h and fused:
+            self.lib.orc_wrapper_set_fused(h, 1)
         return WrapperContext(self, h, channels, src_bits, dst_bits) if h else None
 
     # ---- Q15 helpers ----
@@ -321,6 +333,12 @@ class Oracle(_Backend):
         self.lib.orc_wrapper_policy.restype = _i
         self.lib.orc_wrapper_policy.argtypes = [_vp, _f32p, C.POINTER(C.c_float), C.POINTER(C.c_float),
                                                 C.POINTER(C.c_int)]
+        for fn in (self.lib.orc_resample_set_fused, self.lib.orc_wrapper_set_fused):
+            fn.restype = None
+            fn.argtypes = [_vp, _i]
+
+    def _check_fused(self, fused):
+        pass
 
     def wrapper_policy(self, w):
         coeffs = np.zeros(5, np.float32)
@@ -356,3 +374,15 @@ def have_reference():
 
 # Synthetic signals (SURVEY.md §8d) live in tests/signals.py (no oracle involved); re-exported for the tests.
 from signals import multitone, noise  # noqa: E402,F401
+
+DYADIC_K = (-14, 0)  # exponents of dyadic(): every bank entry times 2^k stays a normal float32
+
+
+def dyadic(frames, channels, stream, kmin=DYADIC_K[0], kmax=DYADIC_K[1]):
+    """Interleaved float32 samples s * 2^k, s in {-1, -0, +0, +1}, k in [kmin, kmax], seeded by `stream`.  Every
+    product of such a sample with a filter tap is exact in FP32, so a multiply-add rounds the same fused or not: on
+    this input the fused (fast-mode) and plain (exact-mode) dot products give the same bits."""
+    rng = np.random.default_rng(0xD1AD1C + stream)
+    n = frames * channels
+    s = rng.choice(np.array([-1.0, -0.0, 0.0, 1.0]), size=n, p=[0.4, 0.1, 0.1, 0.4])
+    return (s * np.ldexp(1.0, rng.integers(kmin, kmax + 1, size=n))).astype(np.float32)
