@@ -29,6 +29,14 @@ static std::atomic<uint64_t> g_launches{0};
 
 namespace espb {
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
+int grid_y_max() {
+  static const int v = [] {
+    const char *s = getenv("ESPB_GRID_Y_MAX");
+    const long n = s ? atol(s) : kMaxGridY;
+    return (int) (n < 1 ? 1 : (n > kMaxGridY ? kMaxGridY : n));
+  }();
+  return v;
+}
 }  // namespace espb
 
 static int fail(int code, const char *what, const char *detail = nullptr) {

@@ -98,20 +98,20 @@ __device__ __forceinline__ float section_step(Section &s, float x, const BiquadP
 }
 
 // src/dst: first group of the launch (may be the same buffer when there is one time block); rows
-// [row_first, row_first + n_rows) of every group are filtered.  blockIdx.y = time block of block_rows rows
-// (0 = all rows in one block) preceded by warm_rows rows of warm-up.
+// [row_first, row_first + n_rows) of every group are filtered.  blk_first + blockIdx.y = time block of block_rows rows
+// (0 = all rows in one block) preceded by warm_rows rows of warm-up; n_blocks = time blocks of the whole call.
 template <int NSEC, bool FIRST_ORDER>
 __global__ void __launch_bounds__(SGN)
     espb_biquad_tm_kernel(const float *src, float *dst, int64_t rows_cap, int row_first, int n_rows, BiquadParams c,
                           float *__restrict__ state, int n_series, int block_rows, int warm_rows,
-                          float4 *__restrict__ blk_state) {
+                          float4 *__restrict__ blk_state, int blk_first, int n_blocks) {
   extern __shared__ __align__(128) unsigned char bq_smem[];
   float (*ring)[RB][SGN] = reinterpret_cast<float (*)[RB][SGN]>(bq_smem);  // [BSTAGES][RB][SGN]
   uint64_t *full = reinterpret_cast<uint64_t *>(bq_smem + sizeof(float) * BSTAGES * RB * SGN);
   const int tid = threadIdx.x;
   const int q = blockIdx.x * SGN + tid;
   // this CTA's time block: rows [blk_lo, blk_hi), started warm_rows earlier (block 0 starts from the saved state)
-  const int blk = blockIdx.y;
+  const int blk = blk_first + blockIdx.y;
   const int blk_lo = block_rows > 0 ? blk * block_rows : 0;
   const int blk_hi = (block_rows > 0 && blk_lo + block_rows < n_rows) ? blk_lo + block_rows : n_rows;
   const int run_lo = (blk == 0 || blk_lo < warm_rows) ? 0 : blk_lo - warm_rows;
@@ -157,8 +157,9 @@ __global__ void __launch_bounds__(SGN)
   }
   __syncthreads();
 
-  // time-block mode: (start, end) state of block `blk` of this thread's series, for the verify kernel
-  float4 *rec = blk_state ? blk_state + ((size_t) (blockIdx.x * gridDim.y + blk) * NSEC * 2) * SGN + tid : nullptr;
+  // time-block mode: (start, end) state of block `blk` of this thread's series, for the verify kernel (indexed by the
+  // call's block count: a launch may cover only a slice of the blocks)
+  float4 *rec = blk_state ? blk_state + (((size_t) blockIdx.x * n_blocks + blk) * NSEC * 2) * SGN + tid : nullptr;
   for (int k = 0; k < n_chunks; ++k) {
     const int st = k % BSTAGES;
     const int rows = chunk_rows(k);
@@ -429,8 +430,8 @@ __global__ void __launch_bounds__(SGN)
 template <int NSEC>
 __global__ void __launch_bounds__(SGN)
     espb_biquad_chain_check_kernel(const float4 *__restrict__ blk_state, int n_blocks, int n_series,
-                                   unsigned int *__restrict__ group_broken) {
-  const int tid = threadIdx.x, k = blockIdx.y + 1;
+                                   unsigned int *__restrict__ group_broken, int k_first) {
+  const int tid = threadIdx.x, k = k_first + blockIdx.y;  // hand-over from block k - 1 to block k
   if (blockIdx.x * SGN + tid >= n_series)
     return;
   const float4 *rec = blk_state + ((size_t) blockIdx.x * n_blocks * NSEC * 2) * SGN + tid;
@@ -741,7 +742,7 @@ cudaError_t launch_tm(const float *src, float *dst, int64_t rows_cap, int row_fi
                       unsigned int *mismatches, cudaStream_t stream, unsigned int *chain_broken) {
   const int n_blocks = block_rows > 0 ? (n_rows + block_rows - 1) / block_rows : 1;
   float4 *rec = block_rows > 0 ? reinterpret_cast<float4 *>(blk_state) : nullptr;
-  const dim3 grid((n_series + SGN - 1) / SGN, n_blocks);
+  const dim3 grid((n_series + SGN - 1) / SGN);  // groups (time blocks: y, in slices)
   const size_t smem = sizeof(float) * BSTAGES * RB * SGN + BSTAGES * sizeof(uint64_t);
   static PerDeviceOnce once;
   if (once.first()) {
@@ -764,13 +765,24 @@ cudaError_t launch_tm(const float *src, float *dst, int64_t rows_cap, int row_fi
     else
       espb_biquad_tm_few_kernel<NSEC, false><<<ctas, SGN, 0, stream>>>(src, dst, row_first, n_rows, c, state, n_series,
                                                                       lanes, block_rows, warm_rows, n_blocks, rec);
-  } else if (c.first_order)
-    espb_biquad_tm_kernel<NSEC, true><<<grid, SGN, smem, stream>>>(src, dst, rows_cap, row_first, n_rows, c, state,
-                                                                   n_series, block_rows, warm_rows, rec);
-  else
-    espb_biquad_tm_kernel<NSEC, false><<<grid, SGN, smem, stream>>>(src, dst, rows_cap, row_first, n_rows, c, state,
-                                                                    n_series, block_rows, warm_rows, rec);
-  count_launch();
+    count_launch();
+  } else {  // time blocks ride on y
+    cudaError_t e = for_each_y_slice(n_blocks, [&](int b0, int nb) {
+      const dim3 grid_b(grid.x, nb);
+      if (c.first_order)
+        espb_biquad_tm_kernel<NSEC, true><<<grid_b, SGN, smem, stream>>>(src, dst, rows_cap, row_first, n_rows, c,
+                                                                         state, n_series, block_rows, warm_rows, rec,
+                                                                         b0, n_blocks);
+      else
+        espb_biquad_tm_kernel<NSEC, false><<<grid_b, SGN, smem, stream>>>(src, dst, rows_cap, row_first, n_rows, c,
+                                                                          state, n_series, block_rows, warm_rows, rec,
+                                                                          b0, n_blocks);
+      count_launch();
+      return cudaGetLastError();
+    });
+    if (e != cudaSuccess)
+      return e;
+  }
   if (rec) {  // prove (or repair) the block hand-overs and commit the final state
     unsigned int *broken = chain_broken;  // one word per group of this launch; NULL: always walk the chain
     if (broken) {
@@ -778,10 +790,15 @@ cudaError_t launch_tm(const float *src, float *dst, int64_t rows_cap, int row_fi
       if (e != cudaSuccess)
         return e;
     }
-    if (broken && n_blocks > 1) {
-      espb_biquad_chain_check_kernel<NSEC><<<dim3(grid.x, n_blocks - 1), SGN, 0, stream>>>(rec, n_blocks, n_series,
-                                                                                         broken);
-      count_launch();
+    if (broken && n_blocks > 1) {  // the n_blocks - 1 hand-overs ride on y
+      cudaError_t e = for_each_y_slice(n_blocks - 1, [&](int k0, int nk) {
+        espb_biquad_chain_check_kernel<NSEC><<<dim3(grid.x, nk), SGN, 0, stream>>>(rec, n_blocks, n_series, broken,
+                                                                                   k0 + 1);
+        count_launch();
+        return cudaGetLastError();
+      });
+      if (e != cudaSuccess)
+        return e;
     }
     if (c.first_order)
       espb_biquad_verify_kernel<NSEC, true><<<grid.x, SGN, 0, stream>>>(src, dst, rows_cap, row_first, n_rows, c, state,

@@ -206,7 +206,7 @@ int fused_process(EspbResampleGroups *g, const float *in, int64_t in_ss, const i
     d.in_off = (int64_t) g->first_stream[k] * in_ss;
     d.n_in = ni;
     d.n_out = gen;
-    d.outs_begin = (int32_t) total_out;
+    d.outs_begin = (int64_t) total_out;
     d.seg_begin = (int32_t) segs.size();
     d.n_segs = (int32_t) f->sched.segs.size();
     d.carry_row = f->carry_row[k];

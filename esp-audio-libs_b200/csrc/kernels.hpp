@@ -11,6 +11,23 @@ namespace espb {
 
 void count_launch();  // bumps the process-wide kernel-launch counter (api.cu)
 
+// CUDA refuses a launch whose gridDim.y exceeds 65,535 (every compute capability).  Launchers that put frames,
+// outputs, time blocks, passes or groups on y enqueue one launch per slice of at most grid_y_max() along y; each
+// kernel takes the slice's first index through an offset it already has (a starting frame or pass, advanced pointers).
+constexpr int kMaxGridY = 65535;
+int grid_y_max();  // kMaxGridY; ESPB_GRID_Y_MAX (read once, clamped to [1, kMaxGridY]) lowers it to test the slicing
+// launch(first, count) for consecutive slices [first, first + count) of [0, total); stops at the first error
+template <class F>
+cudaError_t for_each_y_slice(int64_t total, F &&launch) {
+  const int64_t step = grid_y_max();
+  for (int64_t y0 = 0; y0 < total; y0 += step) {
+    const cudaError_t e = launch((int) y0, (int) (total - y0 < step ? total - y0 : step));
+    if (e != cudaSuccess)
+      return e;
+  }
+  return cudaSuccess;
+}
+
 // Function attributes (dynamic shared-memory size, carve-out) are per device: one flag per device and kernel.
 struct PerDeviceOnce {
   bool done[64] = {};
@@ -92,8 +109,8 @@ struct FsGroupDesc {
   int64_t x_old_off;  // ... inside the previous one (the carried frames)
   int64_t out_off;    // first stream of the group in the caller's output
   int64_t in_off;     // ... in the caller's input
+  int64_t outs_begin;           // first entry of the group in the concatenated schedule
   int32_t n_in, n_out;
-  int32_t outs_begin;           // first entry of the group in the concatenated schedule
   int32_t seg_begin, n_segs;    // its runs in the concatenated segment table
   int32_t carry_row;            // row of the previous staging buffer where the carried frames start
 };

@@ -327,17 +327,11 @@ cudaError_t launch_q2f(const uint8_t *in, int64_t in_row_bytes, float *out, int6
                        uint32_t row_samples, int bits, float gain_factor, cudaStream_t stream) {
   if (rows <= 0 || row_samples == 0)
     return cudaSuccess;
-  constexpr int kMaxGridY = 65535;  // rows ride on gridDim.y: larger batches go in slices
-  if (rows > kMaxGridY) {
-    for (int r0 = 0; r0 < rows; r0 += kMaxGridY) {
-      const int nr = rows - r0 < kMaxGridY ? rows - r0 : kMaxGridY;
-      cudaError_t e = launch_q2f(in + (int64_t) r0 * in_row_bytes, in_row_bytes, out + (int64_t) r0 * out_row_floats,
-                                 out_row_floats, nr, row_samples, bits, gain_factor, stream);
-      if (e != cudaSuccess)
-        return e;
-    }
-    return cudaSuccess;
-  }
+  if (rows > grid_y_max())  // rows ride on gridDim.y: larger batches go in slices
+    return for_each_y_slice(rows, [&](int r0, int nr) {
+      return launch_q2f(in + (int64_t) r0 * in_row_bytes, in_row_bytes, out + (int64_t) r0 * out_row_floats,
+                        out_row_floats, nr, row_samples, bits, gain_factor, stream);
+    });
   const int nbytes = (bits + 7) / 8;
   int vec_ok = ((uintptr_t) in % 4 == 0) && (in_row_bytes % 4 == 0 || rows == 1) &&
                ((uintptr_t) out % 16 == 0) && (out_row_floats % 4 == 0 || rows == 1);
@@ -372,17 +366,12 @@ cudaError_t launch_f2q(const float *in, int64_t in_row_floats, uint8_t *out, int
                        uint32_t row_samples, int bits, uint32_t *clipped, bool clipped_per_row, cudaStream_t stream) {
   if (rows <= 0 || row_samples == 0)
     return cudaSuccess;
-  if (rows > 65535) {  // rows ride on gridDim.y: larger batches go in slices
-    for (int r0 = 0; r0 < rows; r0 += 65535) {
-      const int nr = rows - r0 < 65535 ? rows - r0 : 65535;
-      cudaError_t e = launch_f2q(in + (int64_t) r0 * in_row_floats, in_row_floats, out + (int64_t) r0 * out_row_bytes,
-                                 out_row_bytes, nr, row_samples, bits,
-                                 (clipped && clipped_per_row) ? clipped + r0 : clipped, clipped_per_row, stream);
-      if (e != cudaSuccess)
-        return e;
-    }
-    return cudaSuccess;
-  }
+  if (rows > grid_y_max())  // rows ride on gridDim.y: larger batches go in slices
+    return for_each_y_slice(rows, [&](int r0, int nr) {
+      return launch_f2q(in + (int64_t) r0 * in_row_floats, in_row_floats, out + (int64_t) r0 * out_row_bytes,
+                        out_row_bytes, nr, row_samples, bits, (clipped && clipped_per_row) ? clipped + r0 : clipped,
+                        clipped_per_row, stream);
+    });
   const int nbytes = (bits + 7) / 8;
   const F2QConst c = make_f2q_const(bits);
   int vec_ok = ((uintptr_t) out % 4 == 0) && (out_row_bytes % 4 == 0 || rows == 1) &&
@@ -423,26 +412,30 @@ int launch_pcm_to_tm(const uint8_t *in, int64_t in_row_bytes, int bits, float ga
   if (fast <= 0 || ((uintptr_t) in % 4) || (in_row_bytes % 4) || n_series <= 0)
     return 0;
   const int nbytes = (bits + 7) / 8;
-  dim3 grid((n_series + SGN - 1) / SGN, fast / PT_ROWS);
-  bool ok = false;
-  switch (nbytes) {
-    case 1:
-      ok = launch_pcm_to_tm_ch<1>(channels, grid, stream, in, in_row_bytes, tm, rows_cap, row_first, n_series, gain_factor);
-      break;
-    case 2:
-      ok = launch_pcm_to_tm_ch<2>(channels, grid, stream, in, in_row_bytes, tm, rows_cap, row_first, n_series, gain_factor);
-      break;
-    case 3:
-      ok = launch_pcm_to_tm_ch<3>(channels, grid, stream, in, in_row_bytes, tm, rows_cap, row_first, n_series, gain_factor);
-      break;
-    case 4:
-      ok = launch_pcm_to_tm_ch<4>(channels, grid, stream, in, in_row_bytes, tm, rows_cap, row_first, n_series, gain_factor);
-      break;
-  }
-  if (!ok)
+  if (nbytes < 1 || nbytes > 4 || !(channels == 1 || channels == 2 || channels == 4 || channels == 8))
     return 0;
-  count_launch();
-  *err = cudaGetLastError();
+  // tiles of frames ride on y: a slice starting at tile y0 reads from frame y0 * PT_ROWS on
+  *err = for_each_y_slice(fast / PT_ROWS, [&](int y0, int ny) {
+    const dim3 grid((n_series + SGN - 1) / SGN, ny);
+    const uint8_t *in_y = in + (int64_t) y0 * PT_ROWS * channels * nbytes;
+    const int row_y = row_first + y0 * PT_ROWS;
+    switch (nbytes) {
+      case 1:
+        launch_pcm_to_tm_ch<1>(channels, grid, stream, in_y, in_row_bytes, tm, rows_cap, row_y, n_series, gain_factor);
+        break;
+      case 2:
+        launch_pcm_to_tm_ch<2>(channels, grid, stream, in_y, in_row_bytes, tm, rows_cap, row_y, n_series, gain_factor);
+        break;
+      case 3:
+        launch_pcm_to_tm_ch<3>(channels, grid, stream, in_y, in_row_bytes, tm, rows_cap, row_y, n_series, gain_factor);
+        break;
+      default:
+        launch_pcm_to_tm_ch<4>(channels, grid, stream, in_y, in_row_bytes, tm, rows_cap, row_y, n_series, gain_factor);
+        break;
+    }
+    count_launch();
+    return cudaGetLastError();
+  });
   return fast;
 }
 
@@ -455,27 +448,31 @@ int launch_tm_to_pcm(const float *tm, int64_t rows_cap, int row_first, int n_fra
   if (fast <= 0 || ((uintptr_t) out % 4) || (out_row_bytes % 4) || n_series <= 0)
     return 0;
   const int nbytes = (bits + 7) / 8;
-  const F2QConst c = make_f2q_const(bits);
-  dim3 grid((n_series + SGN - 1) / SGN, fast / PT_ROWS);
-  bool ok = false;
-  switch (nbytes) {
-    case 1:
-      ok = launch_tm_to_pcm_ch<1>(channels, grid, stream, tm, rows_cap, row_first, out, out_row_bytes, n_series, c, clipped_per_stream);
-      break;
-    case 2:
-      ok = launch_tm_to_pcm_ch<2>(channels, grid, stream, tm, rows_cap, row_first, out, out_row_bytes, n_series, c, clipped_per_stream);
-      break;
-    case 3:
-      ok = launch_tm_to_pcm_ch<3>(channels, grid, stream, tm, rows_cap, row_first, out, out_row_bytes, n_series, c, clipped_per_stream);
-      break;
-    case 4:
-      ok = launch_tm_to_pcm_ch<4>(channels, grid, stream, tm, rows_cap, row_first, out, out_row_bytes, n_series, c, clipped_per_stream);
-      break;
-  }
-  if (!ok)
+  if (nbytes < 1 || nbytes > 4 || !(channels == 1 || channels == 2 || channels == 4 || channels == 8))
     return 0;
-  count_launch();
-  *err = cudaGetLastError();
+  const F2QConst c = make_f2q_const(bits);
+  // tiles of frames ride on y: a slice starting at tile y0 writes from frame y0 * PT_ROWS on
+  *err = for_each_y_slice(fast / PT_ROWS, [&](int y0, int ny) {
+    const dim3 grid((n_series + SGN - 1) / SGN, ny);
+    const int row_y = row_first + y0 * PT_ROWS;
+    uint8_t *out_y = out + (int64_t) y0 * PT_ROWS * channels * nbytes;
+    switch (nbytes) {
+      case 1:
+        launch_tm_to_pcm_ch<1>(channels, grid, stream, tm, rows_cap, row_y, out_y, out_row_bytes, n_series, c, clipped_per_stream);
+        break;
+      case 2:
+        launch_tm_to_pcm_ch<2>(channels, grid, stream, tm, rows_cap, row_y, out_y, out_row_bytes, n_series, c, clipped_per_stream);
+        break;
+      case 3:
+        launch_tm_to_pcm_ch<3>(channels, grid, stream, tm, rows_cap, row_y, out_y, out_row_bytes, n_series, c, clipped_per_stream);
+        break;
+      default:
+        launch_tm_to_pcm_ch<4>(channels, grid, stream, tm, rows_cap, row_y, out_y, out_row_bytes, n_series, c, clipped_per_stream);
+        break;
+    }
+    count_launch();
+    return cudaGetLastError();
+  });
   return fast;
 }
 

@@ -380,11 +380,14 @@ cudaError_t launch_fsg_stage(const FsGroupDesc *groups, int n_groups, const floa
   // about 2048 elements per CTA
   int rows_per_cta = 2048 / pitch;
   rows_per_cta = rows_per_cta < 1 ? 1 : rows_per_cta;
-  const dim3 grid((max_rows + rows_per_cta - 1) / rows_per_cta, n_groups);
-  espb_fsg_stage_kernel<<<grid, 256, 0, stream>>>(groups, old_buf, new_buf, pitch, taps, in, in_ss, channels, n_series,
-                                                  rows_per_cta);
-  count_launch();
-  return cudaGetLastError();
+  // groups ride on y: a slice takes the descriptors from its first group on (their offsets are absolute)
+  return for_each_y_slice(n_groups, [&](int g0, int ng) {
+    const dim3 grid((max_rows + rows_per_cta - 1) / rows_per_cta, ng);
+    espb_fsg_stage_kernel<<<grid, 256, 0, stream>>>(groups + g0, old_buf, new_buf, pitch, taps, in, in_ss, channels,
+                                                    n_series, rows_per_cta);
+    count_launch();
+    return cudaGetLastError();
+  });
 }
 
 cudaError_t launch_expand_schedule_groups(const FsGroupDesc *groups, int n_groups, const SchedSegment *segs,
@@ -392,10 +395,13 @@ cudaError_t launch_expand_schedule_groups(const FsGroupDesc *groups, int n_group
                                           cudaStream_t stream) {
   if (n_groups <= 0 || max_n_out <= 0)
     return cudaSuccess;
-  const dim3 grid((max_n_out + 255) / 256, n_groups);
-  espb_expand_schedule_groups_kernel<<<grid, 256, 0, stream>>>(groups, segs, outs, (float) n_filters, lowpass, interp);
-  count_launch();
-  return cudaGetLastError();
+  return for_each_y_slice(n_groups, [&](int g0, int ng) {
+    const dim3 grid((max_n_out + 255) / 256, ng);
+    espb_expand_schedule_groups_kernel<<<grid, 256, 0, stream>>>(groups + g0, segs, outs, (float) n_filters, lowpass,
+                                                                 interp);
+    count_launch();
+    return cudaGetLastError();
+  });
 }
 
 // Tap-range width of the slices: the widest power of two (4..64) that divides `taps` and keeps one slice of all
@@ -475,17 +481,23 @@ cudaError_t launch_resample_fs(const FsParams &p_in, const FsGeometry &g, int x_
                   ? 1
                   : 0;
   // (fused groups: n_out is the largest group's count; CTAs past a group's own count leave at once)
-  const dim3 grid((p.n_out + g.outputs_per_cta - 1) / g.outputs_per_cta, p.groups ? n_groups : 1);
+  // (fused groups ride on y: a slice takes the descriptors from its first group on)
+  return for_each_y_slice(p.groups ? n_groups : 1, [&](int g0, int ng) {
+    FsParams pg = p;
+    if (p.groups)
+      pg.groups = p.groups + g0;
+    const dim3 grid((p.n_out + g.outputs_per_cta - 1) / g.outputs_per_cta, ng);
 #define ESPB_FS(SV_, B_) \
-  (exact ? launch_fs_t<SV_, B_, true>(p, smem, grid, stream) : launch_fs_t<SV_, B_, false>(p, smem, grid, stream))
-  if (g.sv == 2 && g.b == 4)
-    return ESPB_FS(2, 4);
-  if (g.sv == 4 && g.b == 4)
-    return ESPB_FS(4, 4);
-  if (g.sv == 8 && g.b == 2)
-    return ESPB_FS(8, 2);
+  (exact ? launch_fs_t<SV_, B_, true>(pg, smem, grid, stream) : launch_fs_t<SV_, B_, false>(pg, smem, grid, stream))
+    if (g.sv == 2 && g.b == 4)
+      return ESPB_FS(2, 4);
+    if (g.sv == 4 && g.b == 4)
+      return ESPB_FS(4, 4);
+    if (g.sv == 8 && g.b == 2)
+      return ESPB_FS(8, 2);
 #undef ESPB_FS
-  return cudaErrorInvalidValue;
+    return cudaErrorInvalidValue;
+  });
 }
 
 }  // namespace espb

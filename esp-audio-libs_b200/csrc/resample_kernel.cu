@@ -435,10 +435,10 @@ __global__ void __launch_bounds__(256)
 // as the generic kernel (frames contiguous per plane: a warp reads 32 consecutive frames of one plane).
 __global__ void __launch_bounds__(256)
     espb_transpose_ptr_kernel(const float *const *__restrict__ planes, int n_series, int n_in,
-                              float *__restrict__ xt, int64_t rows_cap, int row_first, int pad_rows) {
+                              float *__restrict__ xt, int64_t rows_cap, int row_first, int j_begin, int pad_rows) {
   __shared__ float tile[TR_ROWS][SGN + 1];
   const int g = blockIdx.x;
-  const int j0 = blockIdx.y * TR_ROWS;
+  const int j0 = j_begin + blockIdx.y * TR_ROWS;
   const int tid = threadIdx.x;
   const int total_rows = n_in + pad_rows;
   for (int i = tid; i < SGN * TR_ROWS; i += 256) {
@@ -459,11 +459,11 @@ __global__ void __launch_bounds__(256)
 }
 
 __global__ void __launch_bounds__(256)
-    espb_untranspose_ptr_kernel(const float *__restrict__ tm, int64_t rows_cap, int row_first, int n_rows,
-                                float *const *__restrict__ planes, int n_series) {
+    espb_untranspose_ptr_kernel(const float *__restrict__ tm, int64_t rows_cap, int row_first, int j_begin,
+                                int n_rows, float *const *__restrict__ planes, int n_series) {
   __shared__ float tile[TR_ROWS][SGN + 1];
   const int g = blockIdx.x;
-  const int j0 = blockIdx.y * TR_ROWS;
+  const int j0 = j_begin + blockIdx.y * TR_ROWS;
   const int tid = threadIdx.x;
   const float *src = tm + ((int64_t) g * rows_cap + row_first + j0) * SGN;
   for (int i = tid; i < TR_ROWS * SGN; i += 256) {
@@ -929,47 +929,43 @@ cudaError_t launch_transpose(const float *in, int64_t in_ss, int64_t in_cs, int6
     vec = 4;
   else if ((uintptr_t) in % 8 == 0 && in_ss % 2 == 0 && cs_ok2)
     vec = 2;
-  if (n_in >= TF_ROWS) {
-    dim3 grid(n_groups, n_in / TF_ROWS);
-    bool done = true;
-#define ESPB_TR(CH_, PL_)                                                                                          \
-  (vec == 4 ? espb_transpose_fast_kernel<CH_, PL_, 4><<<grid, TF_THREADS, 0, stream>>>(in, in_ss, in_cs, channels,  \
-                                                                                      n_series, xt, rows_cap,     \
-                                                                                      row_first)                  \
-   : vec == 2                                                                                                      \
-       ? espb_transpose_fast_kernel<CH_, PL_, 2><<<grid, TF_THREADS, 0, stream>>>(in, in_ss, in_cs, channels,       \
-                                                                                 n_series, xt, rows_cap, row_first) \
-       : espb_transpose_fast_kernel<CH_, PL_, 1><<<grid, TF_THREADS, 0, stream>>>(in, in_ss, in_cs, channels,       \
-                                                                                 n_series, xt, rows_cap, row_first))
-    if (interleaved && channels == 1)
-      ESPB_TR(1, false);
-    else if (interleaved && channels == 2)
-      ESPB_TR(2, false);
-    else if (interleaved && channels == 4)
-      ESPB_TR(4, false);
-    else if (interleaved && channels == 8)
-      ESPB_TR(8, false);
-    else if (planar)
-      ESPB_TR(1, true);
-    else
-      done = false;
+  const bool fast_layout = (interleaved && (channels == 1 || channels == 2 || channels == 4 || channels == 8)) || planar;
+  if (n_in >= TF_ROWS && fast_layout) {
+    // a slice starting at tile y0 reads from frame y0 * TF_ROWS on (in_fs = channels or 1 here) and writes the rows
+    // from row_first + y0 * TF_ROWS on
+    cudaError_t e = for_each_y_slice(n_in / TF_ROWS, [&](int y0, int ny) {
+      const dim3 grid(n_groups, ny);
+      const float *in_y = in + (int64_t) y0 * TF_ROWS * in_fs;
+      const int row_y = row_first + y0 * TF_ROWS;
+#define ESPB_TR(CH_, PL_)                                                                                             \
+  (vec == 4 ? espb_transpose_fast_kernel<CH_, PL_, 4><<<grid, TF_THREADS, 0, stream>>>(in_y, in_ss, in_cs, channels,   \
+                                                                                      n_series, xt, rows_cap, row_y)   \
+   : vec == 2                                                                                                         \
+       ? espb_transpose_fast_kernel<CH_, PL_, 2><<<grid, TF_THREADS, 0, stream>>>(in_y, in_ss, in_cs, channels,        \
+                                                                                 n_series, xt, rows_cap, row_y)        \
+       : espb_transpose_fast_kernel<CH_, PL_, 1><<<grid, TF_THREADS, 0, stream>>>(in_y, in_ss, in_cs, channels,        \
+                                                                                 n_series, xt, rows_cap, row_y))
+      if (interleaved && channels == 1)
+        ESPB_TR(1, false);
+      else if (interleaved && channels == 2)
+        ESPB_TR(2, false);
+      else if (interleaved && channels == 4)
+        ESPB_TR(4, false);
+      else if (interleaved && channels == 8)
+        ESPB_TR(8, false);
+      else
+        ESPB_TR(1, true);
 #undef ESPB_TR
-    if (done) {
       count_launch();
-      fast_rows = (n_in / TF_ROWS) * TF_ROWS;
-      cudaError_t e = cudaGetLastError();
-      if (e != cudaSuccess)
-        return e;
-    }
+      return cudaGetLastError();
+    });
+    if (e != cudaSuccess)
+      return e;
+    fast_rows = (n_in / TF_ROWS) * TF_ROWS;
   }
-  const int rest = n_in + pad_rows - fast_rows;
-  if (rest > 0) {
-    dim3 grid(n_groups, (rest + TR_ROWS - 1) / TR_ROWS);
-    espb_transpose_kernel<<<grid, 256, 0, stream>>>(in, in_ss, in_cs, in_fs, channels, n_series, n_in, xt, rows_cap,
-                                                    row_first, fast_rows, pad_rows);
-    count_launch();
-  }
-  return cudaGetLastError();
+  cudaError_t e = launch_transpose_from(in, in_ss, in_cs, in_fs, channels, n_series, n_in, xt, rows_cap, row_first,
+                                        fast_rows, pad_rows, stream);
+  return e != cudaSuccess ? e : cudaGetLastError();
 }
 
 // The staging of a long call arranged for overlap with the resampler (see espb_transpose_flags_kernel): everything
@@ -988,14 +984,11 @@ cudaError_t launch_transpose_flags(const float *in, int64_t in_ss, int64_t in_cs
   if (n_groups <= 0 || n_in < kReadyTileRows || !covered || (uintptr_t) in % 16 != 0 || in_ss % 4 != 0 || !cs_ok4)
     return cudaSuccess;
   const int tiles_y = n_in / kReadyTileRows, fast_rows = tiles_y * kReadyTileRows;
-  const int rest = n_in + pad_rows - fast_rows;
-  if (rest > 0) {
-    dim3 grid(n_groups, (rest + TR_ROWS - 1) / TR_ROWS);
-    espb_transpose_kernel<<<grid, 256, 0, stream>>>(in, in_ss, in_cs, in_fs, channels, n_series, n_in, xt, rows_cap,
-                                                    row_first, fast_rows, pad_rows);
-    count_launch();
-  }
-  cudaError_t e = cudaMemsetAsync(ready, 0, (size_t) tiles_y * sizeof(int), stream);
+  cudaError_t e = launch_transpose_from(in, in_ss, in_cs, in_fs, channels, n_series, n_in, xt, rows_cap, row_first,
+                                        fast_rows, pad_rows, stream);
+  if (e != cudaSuccess)
+    return e;
+  e = cudaMemsetAsync(ready, 0, (size_t) tiles_y * sizeof(int), stream);
   if (e != cudaSuccess)
     return e;
   int sms = 148, dev = 0;
@@ -1064,10 +1057,12 @@ cudaError_t launch_transpose_ptrs(const float *const *planes_dev, int n_series, 
   const int n_groups = (n_series + SGN - 1) / SGN;
   if (n_groups <= 0 || n_in + pad_rows <= 0)
     return cudaSuccess;
-  dim3 grid(n_groups, (n_in + pad_rows + TR_ROWS - 1) / TR_ROWS);
-  espb_transpose_ptr_kernel<<<grid, 256, 0, stream>>>(planes_dev, n_series, n_in, xt, rows_cap, row_first, pad_rows);
-  count_launch();
-  return cudaGetLastError();
+  return for_each_y_slice((n_in + pad_rows + TR_ROWS - 1) / TR_ROWS, [&](int y0, int ny) {
+    espb_transpose_ptr_kernel<<<dim3(n_groups, ny), 256, 0, stream>>>(planes_dev, n_series, n_in, xt, rows_cap,
+                                                                      row_first, y0 * TR_ROWS, pad_rows);
+    count_launch();
+    return cudaGetLastError();
+  });
 }
 
 cudaError_t launch_untranspose_ptrs(const float *tm, int64_t rows_cap, int row_first, int n_rows,
@@ -1075,10 +1070,12 @@ cudaError_t launch_untranspose_ptrs(const float *tm, int64_t rows_cap, int row_f
   const int n_groups = (n_series + SGN - 1) / SGN;
   if (n_groups <= 0 || n_rows <= 0)
     return cudaSuccess;
-  dim3 grid(n_groups, (n_rows + TR_ROWS - 1) / TR_ROWS);
-  espb_untranspose_ptr_kernel<<<grid, 256, 0, stream>>>(tm, rows_cap, row_first, n_rows, planes_dev, n_series);
-  count_launch();
-  return cudaGetLastError();
+  return for_each_y_slice((n_rows + TR_ROWS - 1) / TR_ROWS, [&](int y0, int ny) {
+    espb_untranspose_ptr_kernel<<<dim3(n_groups, ny), 256, 0, stream>>>(tm, rows_cap, row_first, y0 * TR_ROWS, n_rows,
+                                                                        planes_dev, n_series);
+    count_launch();
+    return cudaGetLastError();
+  });
 }
 
 // generic kernels only, starting at frame j_begin (used for the tails after the fused PCM tiles)
@@ -1089,11 +1086,13 @@ cudaError_t launch_transpose_from(const float *in, int64_t in_ss, int64_t in_cs,
   const int rest = n_in + pad_rows - j_begin;
   if (n_groups <= 0 || rest <= 0)
     return cudaSuccess;
-  dim3 grid(n_groups, (rest + TR_ROWS - 1) / TR_ROWS);
-  espb_transpose_kernel<<<grid, 256, 0, stream>>>(in, in_ss, in_cs, in_fs, channels, n_series, n_in, xt, rows_cap,
-                                                  row_first, j_begin, pad_rows);
-  count_launch();
-  return cudaGetLastError();
+  return for_each_y_slice((rest + TR_ROWS - 1) / TR_ROWS, [&](int y0, int ny) {
+    espb_transpose_kernel<<<dim3(n_groups, ny), 256, 0, stream>>>(in, in_ss, in_cs, in_fs, channels, n_series, n_in, xt,
+                                                                  rows_cap, row_first, j_begin + y0 * TR_ROWS,
+                                                                  pad_rows);
+    count_launch();
+    return cudaGetLastError();
+  });
 }
 
 cudaError_t launch_untranspose_from(const float *tm, int64_t rows_cap, int row_first, int j_begin, int n_rows,
@@ -1103,11 +1102,13 @@ cudaError_t launch_untranspose_from(const float *tm, int64_t rows_cap, int row_f
   const int rest = n_rows - j_begin;
   if (n_groups <= 0 || rest <= 0)
     return cudaSuccess;
-  dim3 grid(n_groups, (rest + TR_ROWS - 1) / TR_ROWS);
-  espb_untranspose_kernel<<<grid, 256, 0, stream>>>(tm, rows_cap, row_first, j_begin, n_rows, out, out_ss, out_cs,
-                                                    out_fs, channels, n_series);
-  count_launch();
-  return cudaGetLastError();
+  return for_each_y_slice((rest + TR_ROWS - 1) / TR_ROWS, [&](int y0, int ny) {
+    espb_untranspose_kernel<<<dim3(n_groups, ny), 256, 0, stream>>>(tm, rows_cap, row_first, j_begin + y0 * TR_ROWS,
+                                                                    n_rows, out, out_ss, out_cs, out_fs, channels,
+                                                                    n_series);
+    count_launch();
+    return cudaGetLastError();
+  });
 }
 
 cudaError_t launch_untranspose(const float *tm, int64_t rows_cap, int row_first, int n_rows, float *out,
@@ -1120,42 +1121,39 @@ cudaError_t launch_untranspose(const float *tm, int64_t rows_cap, int row_first,
   const bool aligned = ((uintptr_t) out % 16 == 0) && (out_ss % 4 == 0);
   const bool interleaved = (out_cs == 1 && out_fs == channels);
   const bool planar = (out_fs == 1) && (out_cs % 4 == 0);
-  if (aligned && n_rows >= TF_ROWS) {
-    dim3 grid(n_groups, n_rows / TF_ROWS);
-    bool done = true;
-    if (interleaved && channels == 1)
-      espb_untranspose_fast_kernel<1, false><<<grid, TF_THREADS, 0, stream>>>(tm, rows_cap, row_first, out, out_ss,
-                                                                              out_cs, channels, n_series);
-    else if (interleaved && channels == 2)
-      espb_untranspose_fast_kernel<2, false><<<grid, TF_THREADS, 0, stream>>>(tm, rows_cap, row_first, out, out_ss,
-                                                                              out_cs, channels, n_series);
-    else if (interleaved && channels == 4)
-      espb_untranspose_fast_kernel<4, false><<<grid, TF_THREADS, 0, stream>>>(tm, rows_cap, row_first, out, out_ss,
-                                                                              out_cs, channels, n_series);
-    else if (interleaved && channels == 8)
-      espb_untranspose_fast_kernel<8, false><<<grid, TF_THREADS, 0, stream>>>(tm, rows_cap, row_first, out, out_ss,
-                                                                              out_cs, channels, n_series);
-    else if (planar)
-      espb_untranspose_fast_kernel<1, true><<<grid, TF_THREADS, 0, stream>>>(tm, rows_cap, row_first, out, out_ss,
-                                                                             out_cs, channels, n_series);
-    else
-      done = false;
-    if (done) {
+  const bool fast_layout = (interleaved && (channels == 1 || channels == 2 || channels == 4 || channels == 8)) || planar;
+  if (aligned && n_rows >= TF_ROWS && fast_layout) {
+    // a slice starting at tile y0 reads the rows from row_first + y0 * TF_ROWS on and writes from frame y0 * TF_ROWS
+    // on (out_fs = channels or 1 here)
+    cudaError_t e = for_each_y_slice(n_rows / TF_ROWS, [&](int y0, int ny) {
+      const dim3 grid(n_groups, ny);
+      const int row_y = row_first + y0 * TF_ROWS;
+      float *out_y = out + (int64_t) y0 * TF_ROWS * out_fs;
+      if (interleaved && channels == 1)
+        espb_untranspose_fast_kernel<1, false><<<grid, TF_THREADS, 0, stream>>>(tm, rows_cap, row_y, out_y, out_ss,
+                                                                                out_cs, channels, n_series);
+      else if (interleaved && channels == 2)
+        espb_untranspose_fast_kernel<2, false><<<grid, TF_THREADS, 0, stream>>>(tm, rows_cap, row_y, out_y, out_ss,
+                                                                                out_cs, channels, n_series);
+      else if (interleaved && channels == 4)
+        espb_untranspose_fast_kernel<4, false><<<grid, TF_THREADS, 0, stream>>>(tm, rows_cap, row_y, out_y, out_ss,
+                                                                                out_cs, channels, n_series);
+      else if (interleaved && channels == 8)
+        espb_untranspose_fast_kernel<8, false><<<grid, TF_THREADS, 0, stream>>>(tm, rows_cap, row_y, out_y, out_ss,
+                                                                                out_cs, channels, n_series);
+      else
+        espb_untranspose_fast_kernel<1, true><<<grid, TF_THREADS, 0, stream>>>(tm, rows_cap, row_y, out_y, out_ss,
+                                                                               out_cs, channels, n_series);
       count_launch();
-      fast_rows = (n_rows / TF_ROWS) * TF_ROWS;
-      cudaError_t e = cudaGetLastError();
-      if (e != cudaSuccess)
-        return e;
-    }
+      return cudaGetLastError();
+    });
+    if (e != cudaSuccess)
+      return e;
+    fast_rows = (n_rows / TF_ROWS) * TF_ROWS;
   }
-  const int rest = n_rows - fast_rows;
-  if (rest > 0) {
-    dim3 grid(n_groups, (rest + TR_ROWS - 1) / TR_ROWS);
-    espb_untranspose_kernel<<<grid, 256, 0, stream>>>(tm, rows_cap, row_first, fast_rows, n_rows, out, out_ss, out_cs,
-                                                      out_fs, channels, n_series);
-    count_launch();
-  }
-  return cudaGetLastError();
+  cudaError_t e = launch_untranspose_from(tm, rows_cap, row_first, fast_rows, n_rows, out, out_ss, out_cs, out_fs,
+                                          channels, n_series, stream);
+  return e != cudaSuccess ? e : cudaGetLastError();
 }
 
 template <int BPP, int NST, int CJ, bool EXACT, bool TMCAP>
@@ -1204,25 +1202,10 @@ static cudaError_t launch_resample_t(const ResampleParams &p, int n_groups, int 
   return cudaGetLastError();
 }
 
-cudaError_t launch_resample(const ResampleParams &p, int bpp, int chunk_rows, bool exact, cudaStream_t stream,
-                            const DirectInput *direct, bool non_interpolating) {
-  const int n_groups = (p.n_series + SGN - 1) / SGN;
-  const int n_passes = p.pass_end - p.pass_first;
-  if (n_groups <= 0 || n_passes <= 0)
-    return cudaSuccess;
-  const int n_ctas_y = (n_passes + p.passes_per_cta - 1) / p.passes_per_cta;
-  const bool tm = p.out_tm != nullptr;
-  ResampleParams q = p;
-  q.out_vec = tm ? kOutVecTimeMajor : kOutVecNone;
-  // 128-bit stores when the caller's layout keeps a lane's results contiguous and aligned
-  if (!tm && (uintptr_t) p.out % 16 == 0 && p.out_ss % 4 == 0) {
-    if (p.out_fs == 1 && (p.out_cs % 4 == 0 || p.channels == 1))  // planar, or mono (no second channel plane)
-      q.out_vec = kOutVecPlanar;
-    else if (p.out_cs == 1 && p.out_fs == p.channels && p.channels == 2)
-      q.out_vec = kOutVecStereo;
-    else if (p.out_cs == 1 && p.out_fs == p.channels && p.channels % 4 == 0)
-      q.out_vec = kOutVecFrame4;
-  }
+// one launch of the resampler over n_ctas_y CTA rows of passes from q.pass_first on
+static cudaError_t launch_resample_slice(const ResampleParams &q, int n_groups, int n_ctas_y, int bpp, int chunk_rows,
+                                         bool exact, bool tm, cudaStream_t stream, const DirectInput *direct,
+                                         bool non_interpolating) {
   // TMCAP: the variant that can also write time-major scratch (kept apart: folding that branch into the
   // caller-layout variant costs it 1.4 % through register allocation)
 #define ESPB_LAUNCH(BPP_, NST_, CJ_)                                                               \
@@ -1254,6 +1237,34 @@ cudaError_t launch_resample(const ResampleParams &p, int bpp, int chunk_rows, bo
     return ESPB_LAUNCH(4, 2, 36);
 #undef ESPB_LAUNCH
   return cudaErrorInvalidValue;
+}
+
+cudaError_t launch_resample(const ResampleParams &p, int bpp, int chunk_rows, bool exact, cudaStream_t stream,
+                            const DirectInput *direct, bool non_interpolating) {
+  const int n_groups = (p.n_series + SGN - 1) / SGN;
+  const int n_passes = p.pass_end - p.pass_first;
+  if (n_groups <= 0 || n_passes <= 0)
+    return cudaSuccess;
+  const int n_ctas_y_total = (n_passes + p.passes_per_cta - 1) / p.passes_per_cta;
+  const bool tm = p.out_tm != nullptr;
+  ResampleParams q = p;
+  q.out_vec = tm ? kOutVecTimeMajor : kOutVecNone;
+  // 128-bit stores when the caller's layout keeps a lane's results contiguous and aligned
+  if (!tm && (uintptr_t) p.out % 16 == 0 && p.out_ss % 4 == 0) {
+    if (p.out_fs == 1 && (p.out_cs % 4 == 0 || p.channels == 1))  // planar, or mono (no second channel plane)
+      q.out_vec = kOutVecPlanar;
+    else if (p.out_cs == 1 && p.out_fs == p.channels && p.channels == 2)
+      q.out_vec = kOutVecStereo;
+    else if (p.out_cs == 1 && p.out_fs == p.channels && p.channels % 4 == 0)
+      q.out_vec = kOutVecFrame4;
+  }
+  // CTAs over passes ride on y: a slice starting at CTA row y0 starts at pass pass_first + y0 * passes_per_cta
+  return for_each_y_slice(n_ctas_y_total, [&](int y0, int n_ctas_y) {
+    ResampleParams qy = q;
+    qy.pass_first = p.pass_first + y0 * p.passes_per_cta;
+    return launch_resample_slice(qy, n_groups, n_ctas_y, bpp, chunk_rows, exact, tm, stream, direct,
+                                 non_interpolating);
+  });
 }
 
 }  // namespace espb

@@ -213,7 +213,10 @@ def test_cpp_shim_compiles_and_links(tmp_path):
 
 @pytest.mark.parametrize("taps,ratio,n_in,split", [(256, 48000 / 44100, 5000, False), (256, 48000 / 44100, 5000, True),
                                                   (64, 0.37, 3001, True), (1024, 44100 / 96000, 9000, True),
-                                                  (32, 3.0, 700, True), (8, 1.0, 100, True)])
+                                                  (32, 3.0, 700, True), (8, 1.0, 100, True),
+                                                  # the call lengths of test_gpu_limits.py's real-size tests
+                                                  (32, 48000 / 44100, 2_100_000, False),
+                                                  (32, 48000 / 44100, 4_200_000, True)])
 def test_pass_plan_covers_every_window(taps, ratio, n_in, split):
     """The chunk table the kernel sweeps (host logic, no GPU): every output's window lies inside the chunks of its
     pass, chunks of a pass are contiguous in time, and the split form the direct-input kernel needs never straddles
@@ -270,6 +273,9 @@ def test_closed_form_schedule_is_the_sequential_machine():
     same(1024, 256, 5, 1024.0, 1024, 960000, 441100, f32(44100) / f32(96000))            # C4 unit
     same(256, 256, 1, 256.0, 256, 480000, 441000, f32(44100) / f32(48000))               # C5 unit
     same(256, 256, 3, 256.0, 256, 160000, 480100, f32(3.0))                              # C3 unit
+    # the call lengths of test_gpu_limits.py's real-size tests (thousands of 16 T ring cycles at T = 32)
+    same(32, 32, 3, 32.0, 32, 2_100_000, 2_290_000, f32(48000) / f32(44100))
+    same(32, 32, 3, 32.0, 32, 4_200_000, 4_580_000, f32(48000) / f32(44100))
     for _ in range(150):
         taps = int(rng.choice([4, 8, 16, 32, 64, 128, 256, 512, 1024, 12, 20, 36, 100, 260]))
         filters, flags = int(rng.integers(2, 1025)), int(rng.integers(0, 8))
