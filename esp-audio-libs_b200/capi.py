@@ -166,7 +166,7 @@ def lib():
                                    C.POINTER(i), vp, vp, vp, vp]),
         "espb_plan_schedule_segments": (i, [i, i, i, f, i, i, i, f, C.POINTER(C.c_uint), C.POINTER(C.c_uint),
                                             C.POINTER(f), C.POINTER(i), vp, vp, vp, vp]),
-        "espb_plan_passes": (i, [i, i, i, f, i, i, i, f, i, i, i, vp, vp, i, vp, i]),
+        "espb_plan_passes": (i, [i, i, i, f, i, i, i, f, i, i, vp, vp, i, vp, i]),
         "espb_plan_policy": (i, [C.POINTER(_Config), C.POINTER(_Coeffs), C.POINTER(f), C.POINTER(f), C.POINTER(i)]),
         "espb_checksum_u32": (i, [vp, u64, vp, vp]),
         "espb_resampleGroupsInit": (vp, [i, C.POINTER(i), i, i, i, f, i]),
@@ -276,17 +276,16 @@ def plan_schedule_segments(taps, filters, flags, offset, index, n_in, n_out, rat
                 ws=ws[:g], phase=ph[:g], w=w[:g], kind=kind[:g], segments=int(rc))
 
 
-def plan_passes(taps, filters, flags, offset, index, n_in, n_out, ratio, blocks_per_pass=4, chunk_rows=32,
-                split_at_zero=False):
+def plan_passes(taps, filters, flags, offset, index, n_in, n_out, ratio, blocks_per_pass=4, chunk_rows=32):
     """Host-only: the chunk table of a call: (chunk_start, chunk_pass, pass_chunk_begin) int32 arrays."""
     n = lib().espb_plan_passes(taps, filters, flags, offset, index, n_in, n_out, ratio, blocks_per_pass, chunk_rows,
-                               int(split_at_zero), None, None, 0, None, 0)
+                               None, None, 0, None, 0)
     if n < 0:
         raise EspbError(f"plan_passes: {_err()}")
     cs, cp = np.zeros(max(n, 1), np.int32), np.zeros(max(n, 1), np.int32)
     pcb = np.zeros(max(n, 1) + 2, np.int32)
     lib().espb_plan_passes(taps, filters, flags, offset, index, n_in, n_out, ratio, blocks_per_pass, chunk_rows,
-                           int(split_at_zero), cs.ctypes.data, cp.ctypes.data, n, pcb.ctypes.data, pcb.size)
+                           cs.ctypes.data, cp.ctypes.data, n, pcb.ctypes.data, pcb.size)
     n_passes = int(cp[n - 1]) + 1 if n else 0
     return cs[:n], cp[:n], pcb[: n_passes + 1]
 

@@ -243,10 +243,10 @@ inline cudaError_t copy_rows_async(void *dst, size_t dpitch, const void *src, si
 
 struct ScheduleKey {
   uint32_t offset_bits = 0, ratio_bits = 0;
-  int index = -1, n_in = -1, n_out = -1, split = 0;
+  int index = -1, n_in = -1, n_out = -1;
   bool operator==(const ScheduleKey &o) const {
     return offset_bits == o.offset_bits && ratio_bits == o.ratio_bits && index == o.index && n_in == o.n_in &&
-           n_out == o.n_out && split == o.split;
+           n_out == o.n_out;
   }
 };
 
@@ -329,8 +329,6 @@ struct EspbResampleBatch {
   float lowpass = 1.0f;
   ArtState state{};
   int mode = ESPB_MODE_FAST;
-  int bpp = 8;  // output blocks (warps) per pass
-  int chunk_rows = 32;  // input rows per pipeline stage (kernel variants: 32 default; 16, 24, 36 selectable)
   std::vector<float> bank_host;
   DevBuf bank;
   // time-major input staging xt[group][row][128]: rows [0, taps) = frames carried over from the
@@ -354,13 +352,11 @@ struct EspbResampleBatch {
   // device staging + CUDA streams of the host-buffer entry point
   DevBuf stage_in, stage_out;
   HostPipe pipe;
-  // direct input (interleaved stereo float, see espb_resample_kernel<..., DIRECT>): decided per call
   // without SUBSAMPLE_INTERPOLATE an output is one dot product: its own kernel and half-size G rows (default geometry)
   bool non_interp = false;
   int g_row_floats() const { return non_interp ? kGRowFloatsNI : kGRowFloats; }
   // output blocks per pass of the plan and of G (the non-interpolating kernel's 4 warps own two blocks each)
-  int plan_bpp() const { return non_interp ? bpp * kNiBlocksPerWarp : bpp; }
-  bool direct_ok = false;    // ESPB_DIRECT=1 switches it on
+  int plan_bpp() const { return non_interp ? kResampleWarps * kNiBlocksPerWarp : kResampleWarps; }
   // few-series form (resample_fs_kernel.cu): lanes own outputs; chosen per context when n_series <= kFsMaxSeries
   int fs_policy = -1;        // ESPB_FS: 0 never, 1 / unset whenever the geometry allows it
   DevBuf bank_tr;            // slice-major copy of the bank
@@ -368,7 +364,6 @@ struct EspbResampleBatch {
   size_t fs_slice = 0;       // floats per slice
   bool fs_call = false;      // this call runs through the few-series kernel (no pass plan, no G)
   int fs_x_rows = 0;         // rows of the widest input tile of a CTA of this call
-  bool direct_call = false;  // this call's plan is split at input frame 0 and its input is read through TMA
   // options
   bool plan_cache = true;   // reuse schedule / tables / G when a call repeats (state, n_in, n_out, ratio)
   bool kernel_timing = false;
@@ -382,7 +377,6 @@ struct EspbResampleBatch {
   bool tables_upload_pending = false;
   // ... so two sets of table storage alternate: a rebuild waits for the upload of the call before the previous one,
   // which in a stream of calls has long finished (no host/device serialisation from call to call)
-  PodBuffer<OutEntry> spare_outs;
   PodBuffer<SchedSegment> spare_segs;
   DevBuf d_ptrs;  // device copy of the plane-pointer tables of espb_resampleProcessPlanes: [2][n_series]
   DevBuf d_segs;
@@ -397,7 +391,6 @@ struct EspbResampleBatch {
   const SchedSegment *p_segs = nullptr;
   const ChunkEntry *p_chunks = nullptr;
   const int32_t *p_pcb = nullptr;
-  bool sched_segments = true;  // closed-form schedule expanded on the device (ESPB_SCHED=seq: per-output host schedule)
   PodBuffer<ChunkEntry> spare_chunks;
   PodBuffer<int32_t> spare_pcb;
   cudaEvent_t spare_uploaded = nullptr;
@@ -432,8 +425,7 @@ void unpin_host_range(void *p) {
 }
 
 // Build (or reuse) the schedule + pass plan for this call and upload the tables.
-int prepare_call(EspbResampleBatch *c, int n_in, int n_out, float ratio, cudaStream_t stream,
-                 bool want_direct = false) {
+int prepare_call(EspbResampleBatch *c, int n_in, int n_out, float ratio, cudaStream_t stream) {
   {
     int dev = -1;
     if (cudaGetDevice(&dev) != cudaSuccess || dev != c->device)
@@ -447,24 +439,17 @@ int prepare_call(EspbResampleBatch *c, int n_in, int n_out, float ratio, cudaStr
     CU_TRY(cudaStreamWaitEvent(stream, c->state_event, 0), "cudaStreamWaitEvent");
     c->state_event_pending = false;
   }
-  // direct input needs the default kernel geometry and a carry that lies inside this call's input
-  want_direct = want_direct && c->direct_ok && !c->non_interp && c->bpp == 4 && c->chunk_rows == 32 &&
-                n_in >= c->geo.taps;
   ScheduleKey k;
   k.offset_bits = f2u(c->state.offset);
   k.ratio_bits = f2u(ratio);
   k.index = c->state.index;
   k.n_in = n_in;
   k.n_out = n_out;
-  k.split = want_direct ? 1 : 0;
-  if (c->plan_cache && c->plan_on_device && k == c->key && c->direct_call == want_direct) {
-    int rc = ensure_xt(c, (int64_t) c->geo.taps + (c->direct_call ? 0 : n_in) + kChunkRows);
-    return rc;
-  }
+  if (c->plan_cache && c->plan_on_device && k == c->key)
+    return ensure_xt(c, (int64_t) c->geo.taps + n_in + kChunkRows);
   c->plan_on_device = false;
   c->g_resident_first = c->g_resident_end = -1;
   {  // rebuild into the storage of the call before the previous one
-    c->sched.outs.swap_storage(c->spare_outs);
     c->sched.segs.swap_storage(c->spare_segs);
     c->plan.chunks.swap_storage(c->spare_chunks);
     c->plan.pass_chunk_begin.swap_storage(c->spare_pcb);
@@ -479,13 +464,8 @@ int prepare_call(EspbResampleBatch *c, int n_in, int n_out, float ratio, cudaStr
     CU_TRY(cudaEventSynchronize(c->tables_uploaded), "cudaEventSynchronize");
     c->tables_upload_pending = false;
   }
-  if (c->sched_segments) {  // a few runs per ring cycle; the per-output entries are expanded on the device
-    build_schedule_segments(c->geo, c->state, n_in, n_out, ratio, c->sched);
-  } else {
-    c->sched.segmented = false;
-    c->sched.segs.clear();
-    build_schedule(c->geo, c->state, n_in, n_out, ratio, c->sched, /*finalize=*/false);  // pass 2 runs on the device
-  }
+  // a few runs per ring cycle; the per-output entries are expanded on the device
+  build_schedule_segments(c->geo, c->state, n_in, n_out, ratio, c->sched);
   c->fs_call = false;
   if (c->bank_tr.p && c->fs_policy != 0 && c->sched.generated > 0) {
     // few-series form: the widest input tile (rows first window .. last window + taps of one CTA's outputs) must fit
@@ -501,12 +481,8 @@ int prepare_call(EspbResampleBatch *c, int n_in, int n_out, float ratio, cudaStr
     c->fs_x_rows = span + c->geo.taps;
     c->fs_call = fs_smem_bytes(fg, c->fs_slice, c->fs_x_rows) <= (size_t) 200 * 1024;
   }
-  if (c->fs_call)
-    want_direct = false;
-  c->direct_call = want_direct && (int) c->sched.used >= c->geo.taps;
-  k.split = c->direct_call ? 1 : 0;
   {
-    int rc = ensure_xt(c, (int64_t) c->geo.taps + (c->direct_call ? 0 : n_in) + kChunkRows);
+    int rc = ensure_xt(c, (int64_t) c->geo.taps + n_in + kChunkRows);
     if (rc != ESPB_OK)
       return rc;
   }
@@ -515,12 +491,11 @@ int prepare_call(EspbResampleBatch *c, int n_in, int n_out, float ratio, cudaStr
     c->plan.pass_chunk_begin.clear();
     c->plan.pass_chunk_begin.push_back(0);
   } else {
-    build_pass_plan(c->sched, c->geo.taps, c->plan_bpp(), c->chunk_rows, c->plan, c->direct_call);
+    build_pass_plan(c->sched, c->geo.taps, c->plan_bpp(), kResampleChunkRows, c->plan);
     // the kernel keeps the chunk table of its passes in shared memory: one pass must fit it.  (32 outputs at a
     // ratio below ~0.004 span more than 320 chunks of input — far outside audio use; refused, not truncated.)
-    const int limit = max_chunks_per_cta(c->bpp, c->chunk_rows);
     for (int ps = 0; ps < c->plan.n_passes(); ++ps)
-      if (c->plan.pass_chunk_begin[ps + 1] - c->plan.pass_chunk_begin[ps] > limit) {
+      if (c->plan.pass_chunk_begin[ps + 1] - c->plan.pass_chunk_begin[ps] > kMaxChunksPerCta) {
         c->key = ScheduleKey{};
         return fail(ESPB_ERR_ARG, "resampleProcess: ratio too small for the kernel's per-pass chunk table");
       }
@@ -531,12 +506,12 @@ int prepare_call(EspbResampleBatch *c, int n_in, int n_out, float ratio, cudaStr
     return ESPB_OK;
   }
   CU_TRY(c->d_outs.reserve((size_t) c->sched.generated * sizeof(OutEntry)), "cudaMalloc schedule");
-  const size_t seg_bytes = c->sched.segmented ? c->sched.segs.size() * sizeof(SchedSegment) : 0;
+  const size_t seg_bytes = c->sched.segs.size() * sizeof(SchedSegment);
   const size_t chunk_bytes = c->fs_call ? 0 : c->plan.chunks.size() * sizeof(ChunkEntry);
   const size_t pcb_bytes = c->fs_call ? 0 : c->plan.pass_chunk_begin.size() * sizeof(int32_t);
   auto up16 = [](size_t v) { return (v + 15) & ~(size_t) 15; };
   const size_t blob_bytes = up16(seg_bytes) + up16(chunk_bytes) + up16(pcb_bytes);
-  if (c->sched.segmented && blob_bytes <= ((size_t) 48 << 10)) {
+  if (blob_bytes <= ((size_t) 48 << 10)) {
     // one upload: the driver copies a pageable source of this size out before cudaMemcpyAsync returns
     CU_TRY(c->d_tables.reserve(blob_bytes + sizeof(ChunkEntry)), "cudaMalloc tables");
     c->h_tables.resize(blob_bytes);
@@ -553,11 +528,9 @@ int prepare_call(EspbResampleBatch *c, int n_in, int n_out, float ratio, cudaStr
   } else {
     CU_TRY(c->d_chunks.reserve((c->plan.chunks.size() + 1) * sizeof(ChunkEntry)), "cudaMalloc chunks");
     CU_TRY(c->d_pcb.reserve(c->plan.pass_chunk_begin.size() * sizeof(int32_t)), "cudaMalloc passes");
-    if (c->sched.segmented) {
-      CU_TRY(c->d_segs.reserve(seg_bytes), "cudaMalloc schedule");
-      CU_TRY(cudaMemcpyAsync(c->d_segs.p, c->sched.segs.data(), seg_bytes, cudaMemcpyHostToDevice, stream),
-             "upload schedule");
-    }
+    CU_TRY(c->d_segs.reserve(seg_bytes), "cudaMalloc schedule");
+    CU_TRY(cudaMemcpyAsync(c->d_segs.p, c->sched.segs.data(), seg_bytes, cudaMemcpyHostToDevice, stream),
+           "upload schedule");
     if (!c->fs_call) {
       CU_TRY(cudaMemcpyAsync(c->d_chunks.p, c->plan.chunks.data(), chunk_bytes, cudaMemcpyHostToDevice, stream),
              "upload chunks");
@@ -568,25 +541,15 @@ int prepare_call(EspbResampleBatch *c, int n_in, int n_out, float ratio, cudaStr
     c->p_chunks = c->d_chunks.as<ChunkEntry>();
     c->p_pcb = c->d_pcb.as<int32_t>();
   }
-  if (c->sched.segmented) {
-    CU_TRY(launch_expand_schedule(c->p_segs, (int) c->sched.segs.size(), c->d_outs.as<OutEntry>(),
-                                  (int) c->sched.generated, c->geo.filters, (c->geo.flags & kFlagLowpass) != 0,
-                                  (c->geo.flags & kFlagInterpolate) != 0, stream),
-           "schedule kernel");
-  } else {
-    CU_TRY(cudaMemcpyAsync(c->d_outs.p, c->sched.outs.data(), c->sched.outs.size() * sizeof(OutEntry),
-                           cudaMemcpyHostToDevice, stream),
-           "upload schedule");
-    CU_TRY(launch_finalize(c->d_outs.as<OutEntry>(), (int) c->sched.outs.size(), c->geo.filters,
-                           (c->geo.flags & kFlagLowpass) != 0, (c->geo.flags & kFlagInterpolate) != 0, stream),
-           "finalize kernel");
-  }
+  CU_TRY(launch_expand_schedule(c->p_segs, (int) c->sched.segs.size(), c->d_outs.as<OutEntry>(),
+                                (int) c->sched.generated, c->geo.filters, (c->geo.flags & kFlagLowpass) != 0,
+                                (c->geo.flags & kFlagInterpolate) != 0, stream),
+         "schedule kernel");
   if (!c->tables_uploaded)
     CU_TRY(cudaEventCreateWithFlags(&c->tables_uploaded, cudaEventDisableTiming), "cudaEventCreate");
   // (pageable tables were copied to a staging area before cudaMemcpyAsync returned: nothing to wait for)
   const size_t pin_from = kPinTablesFrom;
-  if (c->sched.outs.cap * sizeof(OutEntry) >= pin_from || c->sched.segs.cap * sizeof(SchedSegment) >= pin_from ||
-      c->plan.chunks.cap * sizeof(ChunkEntry) >= pin_from ||
+  if (c->sched.segs.cap * sizeof(SchedSegment) >= pin_from || c->plan.chunks.cap * sizeof(ChunkEntry) >= pin_from ||
       c->plan.pass_chunk_begin.cap * sizeof(int32_t) >= pin_from) {
     CU_TRY(cudaEventRecord(c->tables_uploaded, stream), "cudaEventRecord");
     c->tables_upload_pending = true;
@@ -598,7 +561,7 @@ int prepare_call(EspbResampleBatch *c, int n_in, int n_out, float ratio, cudaStr
 // Number of passes per time slab so that the expanded coefficients fit the G budget.
 int passes_per_slab(const EspbResampleBatch *c) {
   const int n_passes = c->plan.n_passes();
-  const size_t chunk_bytes = g_chunk_floats(c->plan_bpp(), c->chunk_rows, c->g_row_floats()) * sizeof(float);
+  const size_t chunk_bytes = g_chunk_floats(c->plan_bpp(), c->g_row_floats()) * sizeof(float);
   const size_t total = c->plan.chunks.size() * chunk_bytes;
   if (total <= c->g_budget_bytes || n_passes <= 1)
     return n_passes;
@@ -611,11 +574,11 @@ int passes_per_slab(const EspbResampleBatch *c) {
 int ensure_g(EspbResampleBatch *c, int chunk_first, int chunk_end, cudaStream_t stream) {
   if (c->g_resident_first == chunk_first && c->g_resident_end == chunk_end)
     return ESPB_OK;
-  const size_t chunk_floats = g_chunk_floats(c->plan_bpp(), c->chunk_rows, c->g_row_floats());
+  const size_t chunk_floats = g_chunk_floats(c->plan_bpp(), c->g_row_floats());
   CU_TRY(c->d_G.reserve((size_t) (chunk_end - chunk_first) * chunk_floats * sizeof(float)), "cudaMalloc G");
   CU_TRY(launch_expand(c->bank.as<float>(), c->d_outs.as<OutEntry>(), c->p_chunks,
                        c->d_G.as<float>(), chunk_first, chunk_end - chunk_first, (int) c->sched.generated,
-                       c->geo.taps, c->plan_bpp(), c->chunk_rows, c->direct_call, stream, c->g_row_floats()),
+                       c->geo.taps, c->plan_bpp(), stream, c->g_row_floats()),
          "expand kernel");
   c->g_resident_first = chunk_first;
   c->g_resident_end = chunk_end;
@@ -629,7 +592,7 @@ int pick_passes_per_cta(const EspbResampleBatch *c, int n_series, int pass_first
   if (cudaGetDevice(&dev) == cudaSuccess)
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const long groups = (n_series + kSeriesPerRow - 1) / kSeriesPerRow;
-  const long slots = (long) sms * (16 / c->bpp);  // resident CTAs
+  const long slots = (long) sms * (16 / kResampleWarps);  // resident CTAs
   // aim for >= 32 waves of CTAs so the tail stays small (measured: 8 waves cost 2.5 %), >= 1 pass per CTA
   long ppc = env_long("ESPB_PPC", 0);
   if (ppc <= 0)
@@ -645,8 +608,8 @@ int pick_passes_per_cta(const EspbResampleBatch *c, int n_series, int pass_first
     if (n > max_chunks)
       max_chunks = n;
   }
-  if (ppc * max_chunks > max_chunks_per_cta(c->bpp, c->chunk_rows))
-    ppc = max_chunks_per_cta(c->bpp, c->chunk_rows) / max_chunks;
+  if (ppc * max_chunks > kMaxChunksPerCta)
+    ppc = kMaxChunksPerCta / max_chunks;
   if (ppc < 1)
     ppc = 1;  // (prepare_call has refused calls in which a single pass is longer than the table)
   return (int) ppc;
@@ -729,46 +692,6 @@ struct StageFilter {
   unsigned int *chain_broken = nullptr;  // one scratch word per group of the range (parallel hand-over check)
 };
 
-// cuTensorMapEncodeTiled through the runtime's driver entry point (the library does not link libcuda, so it still
-// loads on a machine without a driver — where nothing can be computed anyway).
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_tiled_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void *ptr = nullptr;
-    cudaDriverEntryPointQueryResult qr;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qr) == cudaSuccess &&
-        qr == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(ptr);
-  }
-  return fn;
-}
-
-// Can `in` (interleaved float) be read by the resampler kernel directly?  Stereo, 16-byte aligned rows.
-bool direct_input_layout(const EspbResampleBatch *c, const float *in, const EspbLayout &il) {
-  return c->channels == 2 && il.channel_stride == 1 && il.frame_stride == 2 && ((uintptr_t) in % 16) == 0 &&
-         il.stream_stride % 4 == 0 && il.stream_stride > 0 && encode_tiled_fn() != nullptr;
-}
-
-// dim0 = frame x channel floats of a stream, dim1 = stream; box = 16 stereo frames (128 bytes) x 64 streams with the
-// 128-byte swizzle; coordinates outside [0, 2 n_in) x [0, n_streams) read as zero.
-int make_input_map(CUtensorMap *map, const float *in, int64_t stream_stride, int n_in, int n_streams) {
-  const cuuint64_t dims[2] = {(cuuint64_t) n_in * 2, (cuuint64_t) n_streams};
-  const cuuint64_t strides[1] = {(cuuint64_t) stream_stride * sizeof(float)};
-  const cuuint32_t box[2] = {32, (cuuint32_t) (kSeriesPerRow / 2)};
-  const cuuint32_t estr[2] = {1, 1};
-  const CUresult r = encode_tiled_fn()(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float *>(in), dims, strides,
-                                       box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                       CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS)
-    return fail(ESPB_ERR_CUDA, "cuTensorMapEncodeTiled failed");
-  return ESPB_OK;
-}
-
 constexpr int kSmallCallFrames = 4096;  // calls up to this many input frames are staged by one fused kernel
 
 // Stage + resample series [series_first, series_first + n_series) of the batch (series_first is a
@@ -786,21 +709,16 @@ int run_series_range(EspbResampleBatch *c, int series_first, int n_series, const
   const size_t row_bytes = kSeriesPerRow * sizeof(float);
   const float *x_old = c->xt[c->xt_cur].as<float>() + (size_t) g0 * rows * kSeriesPerRow;
   float *x_new = c->xt[1 - c->xt_cur].as<float>() + (size_t) g0 * rows * kSeriesPerRow;
-  // direct input: nothing is staged — the kernel reads the carried frames where they lie and the new frames from
-  // the caller's buffer; afterwards the frames [used - taps, used) become rows [0, taps) of the other buffer
-  const bool direct = c->direct_call && !pre && !post && !pcm_in && !pcm_out && !ptrs;
-  if (c->direct_call && !direct)
-    return fail(ESPB_ERR_STATE, "direct-input plan with library stages around the resampler");
   // real-time chunks of float input: carried frames, transposition and padding in one launch (the three separate
   // operations cost more in launch gaps than in work)
   const bool pre_on_ = pre && pre->params && n_in > 0;
-  const bool small_stage = !direct && !pcm_in && !ptrs && n_in <= kSmallCallFrames &&
+  const bool small_stage = !pcm_in && !ptrs && n_in <= kSmallCallFrames &&
                            !(pre_on_ && pre->block_rows > 0 && n_in > pre->block_rows);
   if (small_stage)
     CU_TRY(launch_stage_small(x_old, c->carry_row, taps, in, il.stream_stride, il.channel_stride, il.frame_stride,
                               c->channels, n_series, n_in, x_new, rows, kChunkRows, stream),
            "staging kernel");
-  else if (!direct)
+  else
     CU_TRY(cudaMemcpy2DAsync(x_new, rows * row_bytes, x_old + (size_t) c->carry_row * kSeriesPerRow, rows * row_bytes,
                              taps * row_bytes, ng, cudaMemcpyDeviceToDevice, stream),
            "carry copy");
@@ -843,9 +761,7 @@ int run_series_range(EspbResampleBatch *c, int series_first, int n_series, const
   const bool pre_on = pre && pre->params && n_in > 0;
   int ready_tiles = 0;  // > 0: the staging kernel just enqueued signals this many row tiles (overlap with the resampler)
   const bool pre_blocks = pre_on && pre->block_rows > 0 && n_in > pre->block_rows;
-  if (direct) {
-    // (no staging)
-  } else if (pre_blocks) {
+  if (pre_blocks) {
     // time-block pre-filter is out of place: the raw frames go to the other staging buffer (its carry rows
     // were copied above, the rest is free), the filter writes the rows the resampler reads
     float *x_raw = c->xt[c->xt_cur].as<float>() + (size_t) g0 * rows * kSeriesPerRow;
@@ -928,15 +844,8 @@ int run_series_range(EspbResampleBatch *c, int series_first, int n_series, const
     ResampleParams p{};
     p.out_tm = y_tm;
     p.out_tm_rows = c->yt_rows;
-    p.xt = direct ? x_old + (size_t) c->carry_row * kSeriesPerRow : x_new;
+    p.xt = x_new;
     p.xt_rows = rows;
-    DirectInput din{};
-    if (direct) {
-      din.in = in;
-      din.in_ss = il.stream_stride;
-      if (int rc = make_input_map(&din.map, in, il.stream_stride, n_in, n_series / c->channels))
-        return rc;
-    }
     p.out = out;
     p.out_ss = ol.stream_stride;
     p.out_cs = ol.channel_stride;
@@ -983,18 +892,10 @@ int run_series_range(EspbResampleBatch *c, int series_first, int n_series, const
         ev_after = c->ev_pool[c->ev_used + 1];
         c->ev_used += 2;
       }
-      CU_TRY(launch_resample(p, c->bpp, c->chunk_rows, c->mode == ESPB_MODE_EXACT, stream, direct ? &din : nullptr,
-                             c->non_interp),
-             "resample kernel");
+      CU_TRY(launch_resample(p, c->mode == ESPB_MODE_EXACT, stream, c->non_interp), "resample kernel");
       if (ev_after)
         CU_TRY(cudaEventRecord(ev_after, stream), "cudaEventRecord");
     }
-  }
-  if (direct) {  // the next call's carry: frames [used - taps, used), time-major, rows [0, taps) of the other buffer
-    const int used = (int) c->sched.used;
-    CU_TRY(launch_transpose(in + (int64_t) (used - taps) * il.frame_stride, il.stream_stride, il.channel_stride,
-                            il.frame_stride, c->channels, n_series, taps, x_new, rows, 0, 0, stream),
-           "carry transpose");
   }
   bool tail_done = false;
   // (worth it for many groups only: the fused kernel's filter warps share their schedulers with the packers and run
@@ -1090,7 +991,7 @@ int ensure_yt(EspbResampleBatch *c, int64_t rows, bool second) {
 void finish_call(EspbResampleBatch *c) {
   // the frames [used - taps, used) of this call are the next call's carry: rows [used, used + taps)
   c->xt_cur = 1 - c->xt_cur;
-  c->carry_row = c->direct_call ? 0 : (int) c->sched.used;  // (direct input: the carry was written to rows [0, taps))
+  c->carry_row = (int) c->sched.used;
   c->state = c->sched.end;
 }
 
@@ -1114,33 +1015,19 @@ EspbResampleBatch *espb_resampleInit(int num_streams, int numChannels, int numTa
   }
   EspbResampleBatch *c = new EspbResampleBatch();
   // page-lock the per-call tables where they are built: their uploads become asynchronous DMA copies
-  c->sched.outs.on_acquire = c->plan.chunks.on_acquire = c->plan.pass_chunk_begin.on_acquire = pin_host_range;
-  c->sched.outs.on_release = c->plan.chunks.on_release = c->plan.pass_chunk_begin.on_release = unpin_host_range;
-  c->spare_outs.on_acquire = c->spare_chunks.on_acquire = c->spare_pcb.on_acquire = pin_host_range;
-  c->spare_outs.on_release = c->spare_chunks.on_release = c->spare_pcb.on_release = unpin_host_range;
+  c->plan.chunks.on_acquire = c->plan.pass_chunk_begin.on_acquire = pin_host_range;
+  c->plan.chunks.on_release = c->plan.pass_chunk_begin.on_release = unpin_host_range;
+  c->spare_chunks.on_acquire = c->spare_pcb.on_acquire = pin_host_range;
+  c->spare_chunks.on_release = c->spare_pcb.on_release = unpin_host_range;
   c->sched.segs.on_acquire = c->spare_segs.on_acquire = pin_host_range;
   c->sched.segs.on_release = c->spare_segs.on_release = unpin_host_range;
-  {
-    const char *sm = getenv("ESPB_SCHED");
-    c->sched_segments = !(sm && strcmp(sm, "seq") == 0);
-  }
   cudaGetDevice(&c->device);
   c->num_streams = num_streams;
   c->channels = numChannels;
   c->geo = ArtGeometry{numTaps, numFilters, flags};
   c->lowpass = lowpassRatio;
   c->state = initial_state(numTaps);
-  // 4 output blocks (warps) per pass, four CTAs per SM: measured 5 % faster than 8 x 2 at C2 (shorter passes
-  // leave less idle time at the pass edges); ESPB_BPP=8 selects the other variant
-  c->bpp = env_long("ESPB_BPP", 4) == 8 ? 8 : 4;
-  {
-    // direct input (no staging pass for interleaved stereo float) is opt-in: measured equal per step at C2 (the kernel
-    // is 8 % slower, the 0.58 ms transposition disappears), it only saves the staging memory
-    c->direct_ok = env_long("ESPB_DIRECT", 0) != 0;
-    const long cr = env_long("ESPB_CHUNK_ROWS", 32);
-    c->chunk_rows = (cr == 16 || ((cr == 24 || cr == 36) && c->bpp == 4)) ? (int) cr : 32;
-  }
-  c->non_interp = (flags & kFlagInterpolate) == 0 && c->bpp == 4 && c->chunk_rows == 32 && env_long("ESPB_NI", 1) != 0;
+  c->non_interp = (flags & kFlagInterpolate) == 0 && env_long("ESPB_NI", 1) != 0;
   long gb = env_long("ESPB_G_MBYTES", 0);
   if (gb > 0)
     c->g_budget_bytes = (size_t) gb << 20;
@@ -1318,8 +1205,7 @@ EspbResampleResult espb_resampleProcessLayout(EspbResampleBatch *c, const float 
   }
   if (numInputFrames < 0)
     numInputFrames = 0;
-  if (prepare_call(c, numInputFrames, numOutputFrames, ratio, as_stream(stream), direct_input_layout(c, in, *il)) !=
-      ESPB_OK)
+  if (prepare_call(c, numInputFrames, numOutputFrames, ratio, as_stream(stream)) != ESPB_OK)
     return res;
   // Long calls: expand the coefficients on a side stream while this stream stages the input (two bandwidth-bound
   // kernels that do not depend on each other); the resampler launch waits for both.
@@ -1393,7 +1279,7 @@ EspbResampleResult espb_resampleProcessPlanes(EspbResampleBatch *c, const float 
   if (numInputFrames < 0)
     numInputFrames = 0;
   cudaStream_t s = as_stream(stream);
-  if (prepare_call(c, numInputFrames, numOutputFrames, ratio, s, false) != ESPB_OK)
+  if (prepare_call(c, numInputFrames, numOutputFrames, ratio, s) != ESPB_OK)
     return res;
   const size_t n = (size_t) c->n_series();
   // the tables are small (8 bytes per plane) and pageable: the driver copies them out before the call returns
@@ -1465,12 +1351,8 @@ EspbResampleResult espb_resampleProcessInterleavedHost(EspbResampleBatch *c, con
       return res;
     }
   }
-  {
-    const EspbLayout stage_layout = {(int64_t) in_row, 1, ch};
-    if (prepare_call(c, numInputFrames, numOutputFrames, ratio, s0,
-                     direct_input_layout(c, hs->stage_in.as<float>(), stage_layout)) != ESPB_OK)
-      return res;
-  }
+  if (prepare_call(c, numInputFrames, numOutputFrames, ratio, s0) != ESPB_OK)
+    return res;
   const size_t out_row = (size_t) c->sched.generated * ch;
   const bool single_slab_g = passes_per_slab(c) >= c->plan.n_passes();
   if (c->sched.generated > 0 && single_slab_g && !c->fs_call) {
@@ -1941,9 +1823,8 @@ int espb_plan_schedule_segments(int numTaps, int numFilters, int flags, float ou
 }
 
 int espb_plan_passes(int numTaps, int numFilters, int flags, float outputOffset, int inputIndex, int numInputFrames,
-                     int numOutputFrames, float ratio, int blocks_per_pass, int chunk_rows, int split_at_zero,
-                     int32_t *chunk_start, int32_t *chunk_pass, int max_chunks, int32_t *pass_chunk_begin,
-                     int max_passes) {
+                     int numOutputFrames, float ratio, int blocks_per_pass, int chunk_rows, int32_t *chunk_start,
+                     int32_t *chunk_pass, int max_chunks, int32_t *pass_chunk_begin, int max_passes) {
   if ((numTaps & 3) || numTaps <= 0 || numTaps > 1024 || numFilters < 2 || numFilters > 1024 || blocks_per_pass <= 0 ||
       chunk_rows <= 0 || chunk_rows > kChunkRows)
     return fail(ESPB_ERR_ARG, "plan_passes: invalid argument");
@@ -1951,7 +1832,7 @@ int espb_plan_passes(int numTaps, int numFilters, int flags, float outputOffset,
   build_schedule(ArtGeometry{numTaps, numFilters, flags}, ArtState{outputOffset, inputIndex}, numInputFrames,
                  numOutputFrames, ratio, s);
   PassPlan plan;
-  build_pass_plan(s, numTaps, blocks_per_pass, chunk_rows, plan, split_at_zero != 0);
+  build_pass_plan(s, numTaps, blocks_per_pass, chunk_rows, plan);
   const int n_chunks = (int) plan.chunks.size(), n_passes = plan.n_passes();
   for (int i = 0; i < n_chunks && i < max_chunks; ++i) {
     if (chunk_start)

@@ -6,21 +6,17 @@ namespace espb {
 
 // Tile geometry of the resampler kernel (see DESIGN.md "Resampler kernel").
 constexpr int kOutputsPerBlock = 8;   // NB: outputs accumulated per thread
-constexpr int kChunkRows = 40;        // most input frames staged per pipeline stage (the kernel variants use 32 or 16)
+constexpr int kChunkRows = 40;        // zero rows staged after the input (a chunk reads up to 31 rows past a window)
 constexpr int kSeriesPerRow = 128;    // series (stream x channel) per warp row: 32 lanes x 4
 constexpr int kGRowFloats = 2 * kOutputsPerBlock;  // 16 coefficients per (row, output block)
 constexpr int kGRowFloatsNI = kOutputsPerBlock;    // 8 in the non-interpolating form (one filter per output)
 constexpr int kNiBlocksPerWarp = 2;  // ... whose warps own two adjacent blocks each: its pass plan has 8 blocks per pass
-// chunk-table entries a CTA caches in shared memory (fewer for the 4-warp variant: four CTAs share an SM)
-#ifdef __CUDACC__
-#define ESPB_HD __host__ __device__
-#else
-#define ESPB_HD
-#endif
-// (the 24-row, 3-stage variant of the 4-warp kernel leaves only ~1.4 KB for tables next to its ring)
-ESPB_HD constexpr int max_chunks_per_cta(int bpp, int chunk_rows) {
-  return bpp == 8 ? 768 : (chunk_rows == 24 || chunk_rows == 36 ? 120 : 320);
-}
+// The resampler kernels' geometry: 4 warps per CTA (one output block each per pass), four CTAs per SM, input rows
+// streamed in 32-row chunks through a 2-stage shared-memory ring.
+constexpr int kResampleWarps = 4;
+constexpr int kResampleStages = 2;
+constexpr int kResampleChunkRows = 32;
+constexpr int kMaxChunksPerCta = 320;  // chunk-table entries a CTA caches in shared memory
 constexpr int kMaxPassesPerCta = 64;
 
 // What the reference does for one output sample (art_resampler.cpp:421-451).

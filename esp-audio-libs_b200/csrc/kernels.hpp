@@ -1,6 +1,5 @@
 // Launch wrappers for the sm_100a kernels (internal; the public boundary is include/esp_audio_b200.h).
 #pragma once
-#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stddef.h>
 #include <stdint.h>
@@ -63,37 +62,19 @@ struct ResampleParams {
   int ready_tiles, ready_target;
 };
 constexpr int kReadyTileRows = 32;
-// Direct input (interleaved stereo float; resample_direct_kernel.cu): rows j >= 0 come from the caller's buffer
-// through a TMA tensor map (dim0 = frame x channel floats, dim1 = stream; box 32 floats x 64 streams, 128-byte
-// swizzle, zero fill outside).  Kept out of ResampleParams: the standard kernel's register allocation is sensitive
-// to the layout of its parameter block.
-struct DirectInput {
-  const float *in;  // the same buffer, for pass-through outputs
-  int64_t in_ss;    // its stream stride, floats
-  alignas(64) CUtensorMap map;
-};
-struct ResampleDirectParams {
-  ResampleParams p;
-  DirectInput d;
-};
 enum OutVec : int { kOutVecNone = 0, kOutVecPlanar = 1, kOutVecStereo = 2, kOutVecFrame4 = 3, kOutVecTimeMajor = 4 };
 
-size_t resample_smem_bytes(int bpp, int chunk_rows, int g_row_floats = kGRowFloats);
-size_t g_chunk_floats(int bpp, int chunk_rows, int g_row_floats = kGRowFloats);
-cudaError_t launch_finalize(OutEntry *outs, int n, int n_filters, bool lowpass, bool interp, cudaStream_t stream);
+size_t resample_smem_bytes(int bpp, int g_row_floats = kGRowFloats);
+size_t g_chunk_floats(int bpp, int g_row_floats = kGRowFloats);
 cudaError_t launch_expand_schedule(const SchedSegment *segs, int n_segs, OutEntry *outs, int n, int n_filters,
                                    bool lowpass, bool interp, cudaStream_t stream);
 cudaError_t launch_expand(const float *bank, const OutEntry *outs, const ChunkEntry *chunks, float *G,
-                          int chunk_first, int n_chunks, int n_out, int taps, int bpp, int chunk_rows,
-                          bool split_at_zero, cudaStream_t stream, int g_row_floats = kGRowFloats);
-cudaError_t launch_resample(const ResampleParams &p, int bpp, int chunk_rows, bool exact, cudaStream_t stream,
-                            const DirectInput *direct = nullptr, bool non_interpolating = false);
-// non-interpolating form (resample_ni_kernel.cu; BPP 4, 32-row chunks): G rows of kGRowFloatsNI floats
+                          int chunk_first, int n_chunks, int n_out, int taps, int bpp, cudaStream_t stream,
+                          int g_row_floats = kGRowFloats);
+cudaError_t launch_resample(const ResampleParams &p, bool exact, cudaStream_t stream, bool non_interpolating = false);
+// non-interpolating form (resample_ni_kernel.cu): G rows of kGRowFloatsNI floats
 cudaError_t launch_resample_ni(const ResampleParams &q, int n_groups, int n_ctas_y, bool exact, bool tm,
                                cudaStream_t stream);
-// direct-input form (BPP 4, 32-row chunks, caller-layout output); called by launch_resample when p.direct is set
-cudaError_t launch_resample_direct(const ResampleParams &p, const DirectInput &d, int n_groups, int n_ctas_y,
-                                   bool exact, cudaStream_t stream);
 cudaError_t launch_transpose(const float *in, int64_t in_ss, int64_t in_cs, int64_t in_fs, int channels, int n_series,
                              int n_in, float *xt, int64_t rows_cap, int row_first, int pad_rows,
                              cudaStream_t stream);

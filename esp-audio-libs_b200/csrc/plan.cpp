@@ -125,8 +125,7 @@ inline void run_machine(const ArtGeometry &g, ArtState &st, int n_in, int n_out,
 // [0, filters]): truncation is the same value and avoids a libm call per output.
 static inline float floor_nonneg(float v) { return (float) (int) v; }
 
-void build_schedule(const ArtGeometry &g, ArtState start, int n_in, int n_out, float ratio, Schedule &s,
-                    bool finalize) {
+void build_schedule(const ArtGeometry &g, ArtState start, int n_in, int n_out, float ratio, Schedule &s) {
   // Upper bound on the outputs of this call: capacity, and what the input can feed — every output moves the
   // offset by 1/ratio, and the offset can run at most (frames available + what is already buffered) ahead.
   size_t cap = n_out > 0 ? (size_t) n_out : 0;
@@ -139,9 +138,8 @@ void build_schedule(const ArtGeometry &g, ArtState start, int n_in, int n_out, f
   s.outs.clear();
   s.outs.reserve(cap + 1);
   // Pass 1 (sequential, branchy): the state machine records, per output, the offset (in .w) and the ring
-  // rebase folded into a window-start base (in .ws).  Pass 2 (finalize_entries, independent per output; on
-  // the device in the processing path): window start, phase, weight and kind from the offset
-  // (art_resampler.cpp:421-451), written into the same 16-byte entries.
+  // rebase folded into a window-start base (in .ws).  Pass 2 (finalize_entries, independent per output): window
+  // start, phase, weight and kind from the offset (art_resampler.cpp:421-451), written into the same 16-byte entries.
   const int half = g.taps / 2, idx0 = start.index;
   ArtState st = start;
   run_machine(g, st, n_in, n_out, ratio, true, true, &s.used, &s.generated, [&](float off, long long base) {
@@ -151,9 +149,7 @@ void build_schedule(const ArtGeometry &g, ArtState start, int n_in, int n_out, f
     s.outs.push_back(e);  // grows if the bound above was ever too small
   });
   s.end = st;
-  s.raw = !finalize;
-  if (finalize)
-    finalize_entries(g, s.outs.data(), s.outs.size());
+  finalize_entries(g, s.outs.data(), s.outs.size());
 }
 
 void finalize_entries(const ArtGeometry &g, OutEntry *out, size_t n) {
@@ -191,7 +187,6 @@ void build_schedule_segments(const ArtGeometry &g, ArtState start, int n_in, int
   s.outs.clear();
   s.segs.clear();
   s.segmented = true;
-  s.raw = false;
   float off = start.offset;
   int idx = start.index;
   long long base = 0, in_left = n_in > 0 ? n_in : 0, out_left = n_out > 0 ? n_out : 0;
@@ -321,7 +316,7 @@ static inline float segment_offset(const SchedSegment &sg, int j) {
 
 int32_t schedule_ws(const Schedule &s, int k, int *cursor) {
   if (!s.segmented)
-    return s.raw ? s.outs[k].ws + (int32_t) s.outs[k].w : s.outs[k].ws;
+    return s.outs[k].ws;
   int c = cursor ? *cursor : 0;
   const int n = (int) s.segs.size();
   if (c < 0 || c >= n || s.segs[c].n0 > k) {  // not a forward walk: binary search
@@ -367,8 +362,7 @@ unsigned expected_output(const ArtGeometry &g, ArtState st, int n_in, float rati
 }
 
 
-void build_pass_plan(const Schedule &s, int taps, int blocks_per_pass, int chunk_rows, PassPlan &p,
-                     bool split_at_zero) {
+void build_pass_plan(const Schedule &s, int taps, int blocks_per_pass, int chunk_rows, PassPlan &p) {
   const int opp = blocks_per_pass * kOutputsPerBlock;
   const int n = (int) s.generated;
   int cursor = 0;
@@ -387,18 +381,8 @@ void build_pass_plan(const Schedule &s, int taps, int blocks_per_pass, int chunk
   for (int first = 0, pass = 0; first < n; first += opp, ++pass) {
     const int last = (first + opp < n ? first + opp : n) - 1;
     const int j0 = entry_ws(s, first), j1 = entry_ws(s, last) + taps;
-    if (split_at_zero && j0 < 0 && j1 > 0) {
-      const int j0a = -((-j0 + 3) / 4 * 4);  // floor to a multiple of 4: frame 0 then falls on a 4-row group
-      for (int j = j0a; j < 0; j += chunk_rows)
-        p.chunks.push_back(ChunkEntry{j, pass});
-      for (int j = 0; j < j1; j += chunk_rows)
-        p.chunks.push_back(ChunkEntry{j, pass});
-    } else {
-      // (direct input: TMA needs the box to start on a 16-byte boundary of the stream's row = an even stereo frame)
-      const int js = (split_at_zero && j0 > 0) ? (j0 & ~1) : j0;
-      for (int j = js; j < j1; j += chunk_rows)
-        p.chunks.push_back(ChunkEntry{j, pass});
-    }
+    for (int j = j0; j < j1; j += chunk_rows)
+      p.chunks.push_back(ChunkEntry{j, pass});
     p.pass_chunk_begin.push_back((int32_t) p.chunks.size());
   }
 }

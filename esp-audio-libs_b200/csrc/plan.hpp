@@ -90,13 +90,11 @@ struct Schedule {
   bool segmented = false;
   unsigned used = 0, generated = 0;
   ArtState end{};
-  bool raw = false;  // entries still hold (window-start base, offset): finalize_entries() not applied yet
 };
 
 // Data-free run of the resampleProcess state machine (art_resampler.cpp:172-199 /
 // :213-240) that records, per output, the window start / phase / weight / kind.
-void build_schedule(const ArtGeometry &g, ArtState start, int n_in, int n_out, float ratio, Schedule &s,
-                    bool finalize = true);
+void build_schedule(const ArtGeometry &g, ArtState start, int n_in, int n_out, float ratio, Schedule &s);
 // The same schedule in closed form.  The offset is a sequential FP32 accumulator (art_resampler.cpp:195,236), but
 // inside one binade every addition of the same step rounds the same way, so the offsets of consecutive outputs are an
 // exact arithmetic progression until the offset crosses a power of two or the ring is rebased (:175-181).  The host
@@ -109,7 +107,7 @@ void build_schedule_segments(const ArtGeometry &g, ArtState start, int n_in, int
 int32_t schedule_ws(const Schedule &s, int k, int *cursor);
 // host expansion of the segmented form into finalized entries (host API, tests)
 void expand_segments(const ArtGeometry &g, const Schedule &s, OutEntry *out);
-// Second pass of the schedule (host version; espb_finalize_kernel is the device twin).
+// Second pass of the schedule (host version; espb_expand_schedule_kernel has the device twin).
 void finalize_entries(const ArtGeometry &g, OutEntry *entries, size_t n);
 
 unsigned required_samples(const ArtGeometry &g, ArtState st, int n_out, float ratio);  // :257-279
@@ -124,11 +122,7 @@ struct PassPlan {
   PodBuffer<int32_t> pass_chunk_begin;  // n_passes + 1 prefix
   int n_passes() const { return (int) pass_chunk_begin.size() - 1; }
 };
-// split_at_zero: no chunk straddles input frame 0 — a pass that starts in the carried frames sweeps them in chunks
-// that begin on a multiple of 4 rows and then starts over at frame 0 (the kernel's direct-input form reads the two
-// sides from different places).
-void build_pass_plan(const Schedule &s, int taps, int blocks_per_pass, int chunk_rows, PassPlan &p,
-                     bool split_at_zero = false);
+void build_pass_plan(const Schedule &s, int taps, int blocks_per_pass, int chunk_rows, PassPlan &p);
 
 // art_biquad.cpp:16-38 (design in double, stored as float).
 struct BiquadCoeffs {

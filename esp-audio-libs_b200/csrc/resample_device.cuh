@@ -1,7 +1,6 @@
-// Device-side helpers shared by the resampler kernels (resample_kernel.cu, resample_direct_kernel.cu): mbarrier /
+// Device-side helpers shared by the resampler kernels (resample_kernel.cu, resample_ni_kernel.cu): mbarrier /
 // TMA / cp.async wrappers, the packed-FP32 multiply-add, tile constants.  Internal.
 #pragma once
-#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -13,7 +12,7 @@ namespace {
 
 constexpr int NB = kOutputsPerBlock;  // 8
 constexpr int SGN = kSeriesPerRow;    // 128
-constexpr uint32_t kPassDone = 1u << 9, kHistory = 1u << 10;  // rtab flags next to r0 (bits 0-3), r1 (4-7)
+constexpr uint32_t kPassDone = 1u << 9;  // rtab flag next to r0 (bits 0-3), r1 (4-7)
 constexpr int RG = 4;  // rows per skip group / inner unroll
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t) __cvta_generic_to_shared(p); }
@@ -45,15 +44,6 @@ __device__ __forceinline__ void tma_bulk_g2s(void *dst_smem, const void *src, ui
                    smem_u32(dst_smem)),
                "l"(src), "r"(bytes), "r"(smem_u32(bar))
                : "memory");
-}
-
-// TMA tiled copy of one box of a 2-D tensor (global -> shared), completion counted on an mbarrier (SASS: UTMALDG).
-__device__ __forceinline__ void tma_tensor2d_g2s(void *dst_smem, const CUtensorMap *map, int c0, int c1, uint64_t *bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];\n" ::"r"(
-          smem_u32(dst_smem)),
-      "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar))
-      : "memory");
 }
 
 __device__ __forceinline__ void cp_async_16(void *dst_smem, const void *src) {

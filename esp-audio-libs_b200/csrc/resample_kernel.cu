@@ -19,9 +19,9 @@
 //        once per call (espb_expand_kernel) and shared by every CTA.
 // With these, one chunk (32 input rows) of either operand is ONE contiguous 16 KB block.
 //
-// Kernel.  A CTA (BPP warps: 4 by default, four CTAs per SM) owns one group (128 series) and sweeps "passes" of BPP
+// Kernel.  A CTA (4 warps, four CTAs per SM) owns one group (128 series) and sweeps "passes" of 4
 // consecutive output blocks (8 outputs each, one block per warp) over the union of their windows in chunks of 32
-// rows, streamed through a 2-stage shared-memory ring (3 stages for the 8-warp variant) with two TMA bulk copies per
+// rows, streamed through a 2-stage shared-memory ring with two TMA bulk copies per
 // chunk (cp.async.bulk -> mbarrier complete_tx; SASS UBLKCP).  There is no producer warp (a fifth warp would not fit
 // four times per SM next to 128-register consumers): the last warp to finish reading a stage re-arms its mbarrier
 // and issues the refill.  At set-up the CTA builds a table of what each warp does in each chunk (first / last
@@ -45,44 +45,11 @@
 namespace espb {
 
 
-// ---------------------------------------------------------------------------------
-// Second pass of the schedule on the device (twin of plan.cpp:finalize_entries; the same IEEE
-// operations, so the same bits): entries arrive as (window-start base, offset) and leave as
-// (window start, phase, weight, kind) — art_resampler.cpp:421-451.
-// ---------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256)
-    espb_finalize_kernel(OutEntry *__restrict__ outs, int n, float n_filters, int lowpass, int interp) {
-  const int k = blockIdx.x * blockDim.x + threadIdx.x;
-  if (k >= n)
-    return;
-  const float off = outs[k].w;
-  const float fl = (float) (int) off;  // offsets are non-negative: truncation == floor
-  float frac = __fsub_rn(off, fl);
-  OutEntry e;
-  e.ws = outs[k].ws + (int32_t) fl;
-  e.phase = 0;
-  e.w = 0.0f;
-  if (frac == 0.0f && !lowpass) {
-    e.kind = kKindPass;
-  } else if (!interp) {
-    e.kind = kKindSingle;
-    e.phase = (int) __fadd_rn(__fmul_rn(frac, n_filters), 0.5f);
-  } else {
-    frac = __fmul_rn(frac, n_filters);
-    const int i = (int) frac;
-    frac = __fsub_rn(frac, (float) i);
-    e.phase = i;
-    e.w = frac;
-    e.kind = (frac == 0.0f && !lowpass) ? kKindSingle : kKindBlend;
-  }
-  outs[k] = e;
-}
-
 // Segmented schedule -> finalized entries: every output finds its arithmetic-progression run (plan.cpp:
 // build_schedule_segments) by binary search, rebuilds its offset exactly (all terms are multiples of one ulp of the
 // run's binade, so the double-precision product and sum are exact and the conversion back does not round) and
-// finishes it like espb_finalize_kernel.  The host uploads a few hundred bytes per ring cycle instead of 16 bytes
-// per output.
+// finishes it like plan.cpp:finalize_entries (the same IEEE operations, so the same bits).  The host uploads a few
+// hundred bytes per ring cycle instead of 16 bytes per output.
 __global__ void __launch_bounds__(256)
     espb_expand_schedule_kernel(const SchedSegment *__restrict__ segs, int n_segs, OutEntry *__restrict__ outs, int n,
                                 float n_filters, int lowpass, int interp) {
@@ -127,14 +94,15 @@ __global__ void __launch_bounds__(256)
 // entries are warp-uniform; the tile goes through (padded) shared memory and leaves as contiguous 16-byte stores.
 // ---------------------------------------------------------------------------------
 constexpr int kExpandThreads = 256;
-constexpr int kExpandTileFloat4 = 36 * 17 > 32 * 33 ? 36 * 17 : 32 * 33;  // rows x (float4 per row + 1 pad)
+// rows x (float4 per row + 1 pad); a row of either G form is 16 float4: 4 blocks x 16 floats, or 8 blocks x 8
+constexpr int kExpandTileFloat4 = kResampleChunkRows * (kResampleWarps * kGRowFloats / 4 + 1);
 
 __global__ void __launch_bounds__(kExpandThreads)
     espb_expand_kernel(const float *__restrict__ bank, const OutEntry *__restrict__ outs,
                        const ChunkEntry *__restrict__ chunks, float *__restrict__ G, int chunk_first, int n_chunks,
-                       int n_out, int taps, int bpp, int CJ, int split_at_zero, int grf) {
+                       int n_out, int taps, int bpp, int grf) {
+  constexpr int CJ = kResampleChunkRows;
   __shared__ float4 tile[kExpandTileFloat4];
-  // float4 per row: 16 (4 warps per pass) or 32; half of that when a row holds one coefficient per output
   const int quads_per_row = bpp * (grf / 4);
   const bool ni = grf == kGRowFloatsNI;
   const int pitch = quads_per_row + 1;
@@ -155,7 +123,7 @@ __global__ void __launch_bounds__(kExpandThreads)
           if (o < n_out) {
             const OutEntry e = outs[o];
             const int k = j - e.ws;
-            if (k >= 0 && k < taps && e.kind >= kKindSingle && !(split_at_zero && ce.j_start < 0 && j >= 0))
+            if (k >= 0 && k < taps && e.kind >= kKindSingle)
               c0 = __ldg(bank + (size_t) e.phase * taps + k);
           }
           v[h] = c0;
@@ -168,8 +136,7 @@ __global__ void __launch_bounds__(kExpandThreads)
         if (o < n_out) {
           const OutEntry e = outs[o];
           const int k = j - e.ws;
-          // (split plan: a chunk of carried frames stops at input frame 0, the next chunk starts there)
-          if (k >= 0 && k < taps && e.kind >= kKindSingle && !(split_at_zero && ce.j_start < 0 && j >= 0)) {
+          if (k >= 0 && k < taps && e.kind >= kKindSingle) {
             c0 = __ldg(bank + (size_t) e.phase * taps + k);
             if (e.kind == kKindBlend)
               c1 = __ldg(bank + (size_t) (e.phase + 1) * taps + k);
@@ -569,18 +536,19 @@ __global__ void __launch_bounds__(256)
 // ---------------------------------------------------------------------------------
 // Resampler
 // ---------------------------------------------------------------------------------
-// BPP: output blocks (= warps) per pass; NST: ring stages.  <8,3>: two 8-warp CTAs per SM; <4,2>: four 4-warp
-// CTAs per SM (shorter passes: less idle time at the pass edges, twice the x traffic from L2).
+// BPP: output blocks (= warps) per pass; NST: ring stages; CJ: rows per chunk.  Four 4-warp CTAs per SM: measured 5 %
+// faster than two 8-warp CTAs at C2 (shorter passes: less idle time at the pass edges, twice the x traffic from L2).
 // (Results in the caller's layout are written once and never read back, but streaming / evict-first stores are not
 // the answer: __stcs and st.global.L2::cache_hint(evict_first) were both measured 5 % slower — 7.39 against 7.02 ms —
 // a lane's 64 contiguous bytes leave as four 16-byte stores and the hinted forms give up their merging in L2.)
 __device__ __forceinline__ void out_store4(float4 *p, float4 v) { *p = v; }
 
-template <int BPP, int NST, int CJ, bool EXACT, bool TMCAP>
-__global__ void __launch_bounds__(BPP * 32, 16 / BPP) espb_resample_kernel(const ResampleParams p) {
+template <bool EXACT, bool TMCAP>
+__global__ void __launch_bounds__(kResampleWarps * 32, 16 / kResampleWarps) espb_resample_kernel(const ResampleParams p) {
+  constexpr int BPP = kResampleWarps, NST = kResampleStages, CJ = kResampleChunkRows;
   constexpr int NTHREADS = BPP * 32;
   constexpr int STAGES = NST;
-  constexpr int MAXC = max_chunks_per_cta(BPP, CJ);
+  constexpr int MAXC = kMaxChunksPerCta;
   static_assert(kMaxPassesPerCta * BPP * sizeof(int2) <= (size_t) NST * CJ * SGN * sizeof(float), "set-up table");
   constexpr int XS_STAGE = CJ * SGN;                // floats
   constexpr int GS_STAGE = CJ * BPP * kGRowFloats;  // floats
@@ -867,24 +835,14 @@ __global__ void __launch_bounds__(BPP * 32, 16 / BPP) espb_resample_kernel(const
 // ---------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------
-int resample_stages(int bpp, int CJ) { return CJ == 24 ? 3 : (CJ == 36 ? 2 : (bpp == 8 ? 3 : 2) * (32 / CJ)); }
-
-size_t resample_smem_bytes(int bpp, int CJ, int grf) {
-  const int stages = resample_stages(bpp, CJ);
+size_t resample_smem_bytes(int bpp, int grf) {
+  constexpr int stages = kResampleStages, CJ = kResampleChunkRows;
   return (size_t) stages * (CJ * bpp * grf + CJ * SGN) * sizeof(float) + stages * sizeof(uint64_t) +
-         stages * sizeof(uint64_t) + max_chunks_per_cta(bpp, CJ) * (sizeof(int32_t) + bpp * sizeof(uint16_t)) +
+         stages * sizeof(uint64_t) + kMaxChunksPerCta * (sizeof(int32_t) + bpp * sizeof(uint16_t)) +
          (size_t) bpp * NB * sizeof(OutEntry) + 4 * sizeof(int32_t);
 }
 
-size_t g_chunk_floats(int bpp, int CJ, int grf) { return (size_t) CJ * bpp * grf; }
-
-cudaError_t launch_finalize(OutEntry *outs, int n, int n_filters, bool lowpass, bool interp, cudaStream_t stream) {
-  if (n <= 0)
-    return cudaSuccess;
-  espb_finalize_kernel<<<(n + 255) / 256, 256, 0, stream>>>(outs, n, (float) n_filters, lowpass, interp);
-  count_launch();
-  return cudaGetLastError();
-}
+size_t g_chunk_floats(int bpp, int grf) { return (size_t) kResampleChunkRows * bpp * grf; }
 
 cudaError_t launch_expand_schedule(const SchedSegment *segs, int n_segs, OutEntry *outs, int n, int n_filters,
                                    bool lowpass, bool interp, cudaStream_t stream) {
@@ -897,8 +855,8 @@ cudaError_t launch_expand_schedule(const SchedSegment *segs, int n_segs, OutEntr
 }
 
 cudaError_t launch_expand(const float *bank, const OutEntry *outs, const ChunkEntry *chunks, float *G,
-                          int chunk_first, int n_chunks, int n_out, int taps, int bpp, int chunk_rows,
-                          bool split_at_zero, cudaStream_t stream, int grf) {
+                          int chunk_first, int n_chunks, int n_out, int taps, int bpp, cudaStream_t stream,
+                          int grf) {
   if (n_chunks <= 0)
     return cudaSuccess;
   int sms = 148, dev = 0;
@@ -907,7 +865,7 @@ cudaError_t launch_expand(const float *bank, const OutEntry *outs, const ChunkEn
   static const int per_sm = getenv("ESPB_EXPAND_CTAS") ? atoi(getenv("ESPB_EXPAND_CTAS")) : 64;
   const int grid = n_chunks < sms * per_sm ? n_chunks : sms * per_sm;  // (a few chunks per CTA at most)
   espb_expand_kernel<<<grid, kExpandThreads, 0, stream>>>(bank, outs, chunks, G, chunk_first, n_chunks, n_out, taps,
-                                                          bpp, chunk_rows, split_at_zero ? 1 : 0, grf);
+                                                          bpp, grf);
   count_launch();
   return cudaGetLastError();
 }
@@ -1156,27 +1114,27 @@ cudaError_t launch_untranspose(const float *tm, int64_t rows_cap, int row_first,
   return e != cudaSuccess ? e : cudaGetLastError();
 }
 
-template <int BPP, int NST, int CJ, bool EXACT, bool TMCAP>
+template <bool EXACT, bool TMCAP>
 static cudaError_t launch_resample_t(const ResampleParams &p, int n_groups, int n_ctas_y, cudaStream_t stream) {
-  const size_t smem = resample_smem_bytes(BPP, CJ);
+  const size_t smem = resample_smem_bytes(kResampleWarps);
   static PerDeviceOnce once;
   if (once.first()) {
-    cudaError_t e = cudaFuncSetAttribute(espb_resample_kernel<BPP, NST, CJ, EXACT, TMCAP>,
+    cudaError_t e = cudaFuncSetAttribute(espb_resample_kernel<EXACT, TMCAP>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
     if (e != cudaSuccess)
       return e;
-    // two CTAs per SM need the full 228 KB carve-out (the default heuristic sizes it for one)
-    e = cudaFuncSetAttribute(espb_resample_kernel<BPP, NST, CJ, EXACT, TMCAP>, cudaFuncAttributePreferredSharedMemoryCarveout,
+    // four CTAs per SM need the full 228 KB carve-out (the default heuristic sizes it for one)
+    e = cudaFuncSetAttribute(espb_resample_kernel<EXACT, TMCAP>, cudaFuncAttributePreferredSharedMemoryCarveout,
                              (int) cudaSharedmemCarveoutMaxShared);
     if (e != cudaSuccess)
       return e;
     if (getenv("ESPB_DEBUG")) {
       int nb = 0;
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, espb_resample_kernel<BPP, NST, CJ, EXACT, TMCAP>, BPP * 32, smem);
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, espb_resample_kernel<EXACT, TMCAP>, kResampleWarps * 32, smem);
       cudaFuncAttributes fa;
-      cudaFuncGetAttributes(&fa, espb_resample_kernel<BPP, NST, CJ, EXACT, TMCAP>);
-      fprintf(stderr, "[espb] resample<%d,%d,%d,%d,%d>: smem %zu B, %d regs, occupancy %d CTA/SM\n", BPP, NST, CJ,
-              (int) EXACT, (int) TMCAP, smem, fa.numRegs, nb);
+      cudaFuncGetAttributes(&fa, espb_resample_kernel<EXACT, TMCAP>);
+      fprintf(stderr, "[espb] resample<%d,%d>: smem %zu B, %d regs, occupancy %d CTA/SM\n", (int) EXACT, (int) TMCAP,
+              smem, fa.numRegs, nb);
     }
   }
   dim3 grid(n_groups, n_ctas_y);
@@ -1185,7 +1143,7 @@ static cudaError_t launch_resample_t(const ResampleParams &p, int n_groups, int 
     // CTAs start while it runs and synchronise with it through p.ready, not through the stream
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
-    cfg.blockDim = dim3(BPP * 32);
+    cfg.blockDim = dim3(kResampleWarps * 32);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = stream;
     cudaLaunchAttribute attr[1];
@@ -1193,54 +1151,30 @@ static cudaError_t launch_resample_t(const ResampleParams &p, int n_groups, int 
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, espb_resample_kernel<BPP, NST, CJ, EXACT, TMCAP>, p);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, espb_resample_kernel<EXACT, TMCAP>, p);
     count_launch();
     return e != cudaSuccess ? e : cudaGetLastError();
   }
-  espb_resample_kernel<BPP, NST, CJ, EXACT, TMCAP><<<grid, BPP * 32, smem, stream>>>(p);
+  espb_resample_kernel<EXACT, TMCAP><<<grid, kResampleWarps * 32, smem, stream>>>(p);
   count_launch();
   return cudaGetLastError();
 }
 
 // one launch of the resampler over n_ctas_y CTA rows of passes from q.pass_first on
-static cudaError_t launch_resample_slice(const ResampleParams &q, int n_groups, int n_ctas_y, int bpp, int chunk_rows,
-                                         bool exact, bool tm, cudaStream_t stream, const DirectInput *direct,
-                                         bool non_interpolating) {
+static cudaError_t launch_resample_slice(const ResampleParams &q, int n_groups, int n_ctas_y, bool exact, bool tm,
+                                         cudaStream_t stream, bool non_interpolating) {
+  if (non_interpolating)  // one filter per output: resample_ni_kernel.cu
+    return launch_resample_ni(q, n_groups, n_ctas_y, exact, tm, stream);
   // TMCAP: the variant that can also write time-major scratch (kept apart: folding that branch into the
   // caller-layout variant costs it 1.4 % through register allocation)
-#define ESPB_LAUNCH(BPP_, NST_, CJ_)                                                               \
-  (exact ? (tm ? launch_resample_t<BPP_, NST_, CJ_, true, true>(q, n_groups, n_ctas_y, stream)     \
-               : launch_resample_t<BPP_, NST_, CJ_, true, false>(q, n_groups, n_ctas_y, stream))   \
-         : (tm ? launch_resample_t<BPP_, NST_, CJ_, false, true>(q, n_groups, n_ctas_y, stream)    \
-               : launch_resample_t<BPP_, NST_, CJ_, false, false>(q, n_groups, n_ctas_y, stream)))
-  if (non_interpolating) {  // one filter per output: resample_ni_kernel.cu
-    if (bpp != 4 || chunk_rows != 32 || direct)
-      return cudaErrorInvalidValue;
-    return launch_resample_ni(q, n_groups, n_ctas_y, exact, tm, stream);
-  }
-  if (direct) {  // input rows straight from the caller's interleaved-stereo buffer (resample_direct_kernel.cu)
-    if (bpp != 4 || chunk_rows != 32 || tm)
-      return cudaErrorInvalidValue;
-    return launch_resample_direct(q, *direct, n_groups, n_ctas_y, exact, stream);
-  }
-  if (bpp == 8 && chunk_rows == 32)
-    return ESPB_LAUNCH(8, 3, 32);
-  if (bpp == 4 && chunk_rows == 32)
-    return ESPB_LAUNCH(4, 2, 32);
-  if (bpp == 8 && chunk_rows == 16)
-    return ESPB_LAUNCH(8, 6, 16);
-  if (bpp == 4 && chunk_rows == 16)
-    return ESPB_LAUNCH(4, 4, 16);
-  if (bpp == 4 && chunk_rows == 24)
-    return ESPB_LAUNCH(4, 3, 24);
-  if (bpp == 4 && chunk_rows == 36)
-    return ESPB_LAUNCH(4, 2, 36);
-#undef ESPB_LAUNCH
-  return cudaErrorInvalidValue;
+  if (exact)
+    return tm ? launch_resample_t<true, true>(q, n_groups, n_ctas_y, stream)
+              : launch_resample_t<true, false>(q, n_groups, n_ctas_y, stream);
+  return tm ? launch_resample_t<false, true>(q, n_groups, n_ctas_y, stream)
+            : launch_resample_t<false, false>(q, n_groups, n_ctas_y, stream);
 }
 
-cudaError_t launch_resample(const ResampleParams &p, int bpp, int chunk_rows, bool exact, cudaStream_t stream,
-                            const DirectInput *direct, bool non_interpolating) {
+cudaError_t launch_resample(const ResampleParams &p, bool exact, cudaStream_t stream, bool non_interpolating) {
   const int n_groups = (p.n_series + SGN - 1) / SGN;
   const int n_passes = p.pass_end - p.pass_first;
   if (n_groups <= 0 || n_passes <= 0)
@@ -1262,8 +1196,7 @@ cudaError_t launch_resample(const ResampleParams &p, int bpp, int chunk_rows, bo
   return for_each_y_slice(n_ctas_y_total, [&](int y0, int n_ctas_y) {
     ResampleParams qy = q;
     qy.pass_first = p.pass_first + y0 * p.passes_per_cta;
-    return launch_resample_slice(qy, n_groups, n_ctas_y, bpp, chunk_rows, exact, tm, stream, direct,
-                                 non_interpolating);
+    return launch_resample_slice(qy, n_groups, n_ctas_y, exact, tm, stream, non_interpolating);
   });
 }
 

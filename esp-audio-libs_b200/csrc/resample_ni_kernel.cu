@@ -25,7 +25,7 @@ __global__ void __launch_bounds__(BPP * 32, 16 / BPP) espb_resample_ni_kernel(co
   constexpr int NO = NB * WB;           // outputs per warp
   constexpr int NTHREADS = BPP * 32;
   constexpr int STAGES = NST;
-  constexpr int MAXC = max_chunks_per_cta(BPP, CJ);
+  constexpr int MAXC = kMaxChunksPerCta;
   static_assert(kMaxPassesPerCta * BPP * sizeof(int2) <= (size_t) NST * CJ * SGN * sizeof(float), "set-up table");
   constexpr int XS_STAGE = CJ * SGN;       // floats
   constexpr int GS_STAGE = CJ * PB * GRF;  // floats
@@ -303,7 +303,7 @@ __global__ void __launch_bounds__(BPP * 32, 16 / BPP) espb_resample_ni_kernel(co
 // barriers, the chunk tables and the schedule entries of 4 warps x 16 outputs.
 size_t resample_ni_smem_bytes(int warps, int CJ, int stages) {
   return (size_t) stages * ((size_t) CJ * warps * kNiBlocksPerWarp * kGRowFloatsNI + (size_t) CJ * SGN) * sizeof(float) +
-         2 * stages * sizeof(uint64_t) + max_chunks_per_cta(warps, CJ) * (sizeof(int32_t) + warps * sizeof(uint16_t)) +
+         2 * stages * sizeof(uint64_t) + kMaxChunksPerCta * (sizeof(int32_t) + warps * sizeof(uint16_t)) +
          (size_t) warps * kNiBlocksPerWarp * NB * sizeof(OutEntry) + 4 * sizeof(int32_t);
 }
 
@@ -350,14 +350,15 @@ static cudaError_t launch_ni_t(const ResampleParams &p, int n_groups, int n_ctas
   return cudaGetLastError();
 }
 
-// BPP 4, 32-row chunks, 2 stages (the default geometry); q.out_vec is already set by launch_resample
+// q.out_vec is already set by launch_resample
 cudaError_t launch_resample_ni(const ResampleParams &q, int n_groups, int n_ctas_y, bool exact, bool tm,
                                cudaStream_t stream) {
+  constexpr int W = kResampleWarps, NST = kResampleStages, CJ = kResampleChunkRows;
   if (exact)
-    return tm ? launch_ni_t<4, 2, 32, true, true>(q, n_groups, n_ctas_y, stream)
-              : launch_ni_t<4, 2, 32, true, false>(q, n_groups, n_ctas_y, stream);
-  return tm ? launch_ni_t<4, 2, 32, false, true>(q, n_groups, n_ctas_y, stream)
-            : launch_ni_t<4, 2, 32, false, false>(q, n_groups, n_ctas_y, stream);
+    return tm ? launch_ni_t<W, NST, CJ, true, true>(q, n_groups, n_ctas_y, stream)
+              : launch_ni_t<W, NST, CJ, true, false>(q, n_groups, n_ctas_y, stream);
+  return tm ? launch_ni_t<W, NST, CJ, false, true>(q, n_groups, n_ctas_y, stream)
+            : launch_ni_t<W, NST, CJ, false, false>(q, n_groups, n_ctas_y, stream);
 }
 
 }  // namespace espb

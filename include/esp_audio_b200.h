@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define ESPB_ABI_VERSION 1
+#define ESPB_ABI_VERSION 2
 
 /* flags — same bits as include/art_resampler.h:21-23 */
 #define ESPB_SUBSAMPLE_INTERPOLATE 0x1
@@ -324,13 +324,11 @@ int espb_plan_schedule_segments(int numTaps, int numFilters, int flags, float ou
                                 int32_t *window_start, int32_t *phase, float *weight, int32_t *kind);
 /* The kernel-side work list of a call: passes of `blocks_per_pass` x 8 outputs, each swept in chunks of `chunk_rows`
  * input rows starting at chunk_start[] (relative to the call's first input frame; negative = carried frames);
- * pass p owns chunks [pass_chunk_begin[p], pass_chunk_begin[p+1]).  split_at_zero: the form the direct-input kernel
- * needs (no chunk straddles frame 0, chunks at or after it start on even frames).  Returns the number of chunks
+ * pass p owns chunks [pass_chunk_begin[p], pass_chunk_begin[p+1]).  Returns the number of chunks
  * (arrays may be NULL or shorter: nothing is written past max_chunks / max_passes entries), < 0 on bad arguments. */
 int espb_plan_passes(int numTaps, int numFilters, int flags, float outputOffset, int inputIndex, int numInputFrames,
-                     int numOutputFrames, float ratio, int blocks_per_pass, int chunk_rows, int split_at_zero,
-                     int32_t *chunk_start, int32_t *chunk_pass, int max_chunks, int32_t *pass_chunk_begin,
-                     int max_passes);
+                     int numOutputFrames, float ratio, int blocks_per_pass, int chunk_rows, int32_t *chunk_start,
+                     int32_t *chunk_pass, int max_chunks, int32_t *pass_chunk_begin, int max_passes);
 /* Resampler::initialize's decisions (resampler.cpp:38-94) without creating anything:
  * returns 0 none / 1 pre / 2 post filter. */
 int espb_plan_policy(const EspbResamplerConfiguration *config, EspbBiquadCoefficients *coeffs, float *sample_ratio,

@@ -328,11 +328,11 @@ def test_staging_overlap(oracle, overlap):
         assert_fast_path(runs[FAST], runs[EXACT], (ns, ch, overlap))
 
 
-@pytest.mark.parametrize("env", [{"ESPB_G_MBYTES": "1"}, {"ESPB_PPC": "7"}, {"ESPB_SCHED": "seq"}],
-                         ids=["g_slabs", "ppc7", "sched_seq"])
+@pytest.mark.parametrize("env", [{"ESPB_G_MBYTES": "1"}, {"ESPB_PPC": "7"}, {}], ids=["g_slabs", "ppc7", "sched_seq"])
 def test_host_switches(oracle, monkeypatch, env):
     """G made resident in 1 MB time slabs (several resampler launches per call), 7 passes per CTA (a partial last
-    pass range), and the host-built sequential schedule: 150 stereo streams, T = 256, three chained calls."""
+    pass range), and the default host decisions (sched_seq: the closed-form schedule these calls plan must reproduce
+    the oracle's sequential state machine): 150 stereo streams, T = 256, three chained calls."""
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     ns, ch = 150, 2
@@ -369,8 +369,7 @@ def test_full_size_batch(oracle):
     assert_fast_path([got[FAST]], [got[EXACT]], "configs[1]")
 
 
-# ---------------------------------------------------------------- 2. all geometries of the standard kernel (child)
-GEOMETRIES = [(4, 32), (8, 32), (4, 16), (8, 16), (4, 24), (4, 36)]  # (ESPB_BPP, ESPB_CHUNK_ROWS)
+# ---------------------------------------------------------------- 2. both fast instantiations of the standard kernel (child)
 GEO_CALLS = [(4500, 5000), (900, 300), (1202, 1400)]
 GEO_SHAPE = (70, 2, (256, 256, 1.0, 3))  # 140 series: a full 128-series group and a partial one
 WRAP_CALLS = [(4500, 4950), (900, 300), (1202, 1400)]  # 44.1 -> 48 kHz stereo int16: post-filter, time-major output
@@ -420,22 +419,20 @@ def _child_geometries(out_dir):
     x = sigs(ns, sum(c[0] for c in GEO_CALLS), ch, seed=800)
     raw = _wrap_raw()
     saved = {}
-    for bpp, rows in GEOMETRIES:
-        os.environ["ESPB_BPP"], os.environ["ESPB_CHUNK_ROWS"] = str(bpp), str(rows)
-        for mode in (FAST, EXACT):
-            b = batch(ns, ch, geo, mode)
-            for k, (y, u, g) in enumerate(device_chain(b, x, GEO_CALLS, [R48] * 3)):
-                saved[f"{bpp}_{rows}_{mode}_{k}_y"] = y
-                saved[f"{bpp}_{rows}_{mode}_{k}_n"] = np.array([u, g], np.int64)
-            st = b.state()
-            saved[f"{bpp}_{rows}_{mode}_state"] = np.array([st[0], st[1]], np.float64)
-            b.free()
-            r = espb.Resampler(ns, 4500 * 2, 4950 * 2, 44100, 48000, 16, 16, 2, True, True, 256, 256, mode=mode)
-            assert r.policy()["filter"] == "post"
-            for k, (y, u, g, clips) in enumerate(_wrapper_chain(r, raw, 2, 2, WRAP_CALLS, 2.0)):
-                saved[f"w_{bpp}_{rows}_{mode}_{k}_y"] = y
-                saved[f"w_{bpp}_{rows}_{mode}_{k}_res"] = np.concatenate([[u, g], clips]).astype(np.int64)
-            r.free()
+    for mode in (FAST, EXACT):
+        b = batch(ns, ch, geo, mode)
+        for k, (y, u, g) in enumerate(device_chain(b, x, GEO_CALLS, [R48] * 3)):
+            saved[f"{mode}_{k}_y"] = y
+            saved[f"{mode}_{k}_n"] = np.array([u, g], np.int64)
+        st = b.state()
+        saved[f"{mode}_state"] = np.array([st[0], st[1]], np.float64)
+        b.free()
+        r = espb.Resampler(ns, 4500 * 2, 4950 * 2, 44100, 48000, 16, 16, 2, True, True, 256, 256, mode=mode)
+        assert r.policy()["filter"] == "post"
+        for k, (y, u, g, clips) in enumerate(_wrapper_chain(r, raw, 2, 2, WRAP_CALLS, 2.0)):
+            saved[f"w_{mode}_{k}_y"] = y
+            saved[f"w_{mode}_{k}_res"] = np.concatenate([[u, g], clips]).astype(np.int64)
+        r.free()
     np.savez(os.path.join(out_dir, "geo.npz"), **saved)
 
 
@@ -451,16 +448,14 @@ def _load_wrapper_chain(m, key):
     return out
 
 
-def test_all_geometries(oracle, tmp_path):
-    """All six (ESPB_BPP, ESPB_CHUNK_ROWS) geometries in fast mode, on caller-layout output (70 stereo streams, T =
-    256, three chained calls) and on time-major output (the wrapper's post-filter, 16-bit PCM, +2 dB so some samples
-    clip): every fast instantiation resample<BPP, NST, ROWS, 0, TMCAP> — twelve, named by the ESPB_DEBUG report of the
-    child — bit-exact against the fused oracle."""
+def test_fast_instantiations(oracle, tmp_path):
+    """The standard kernel in fast mode on caller-layout output (70 stereo streams, T = 256, three chained calls) and
+    on time-major output (the wrapper's post-filter, 16-bit PCM, +2 dB so some samples clip): both fast
+    instantiations resample<0, TMCAP>, named by the ESPB_DEBUG report of the child, bit-exact against the fused
+    oracle."""
     err = run_child(tmp_path, "_child_geometries", {"ESPB_DEBUG": "1"})
-    seen = set(re.findall(r"\[espb\] resample<(\d+),(\d+),(\d+),0,(\d)>", err))
-    stages = {(4, 32): 2, (8, 32): 3, (4, 16): 4, (8, 16): 6, (4, 24): 3, (4, 36): 2}
-    want = {(str(b), str(stages[(b, r)]), str(r), str(t)) for b, r in GEOMETRIES for t in (0, 1)}
-    assert seen >= want, sorted(want - seen)
+    seen = set(re.findall(r"\[espb\] resample<0,(\d)>", err))
+    assert seen >= {"0", "1"}, sorted(seen)
     m = np.load(tmp_path / "geo.npz")
     ns, ch, geo = GEO_SHAPE
     x = sigs(ns, sum(c[0] for c in GEO_CALLS), ch, seed=800)
@@ -470,19 +465,17 @@ def test_all_geometries(oracle, tmp_path):
     wprobes = (0, 1, 2, 3, 31, 32, 63, 64, 69)
     wref = {s: _oracle_wrapper_chain(oracle, raw[s], 2, 2, 44100, 48000, 16, 16, WRAP_CALLS, 2.0) for s in wprobes}
     assert sum(c[3] for chain in wref.values() for c in chain) > 0  # clip counts were compared
-    for bpp, rows in GEOMETRIES:
-        key = f"{bpp}_{rows}"
-        fast, exact = _load_chain(m, f"{key}_{FAST}"), _load_chain(m, f"{key}_{EXACT}")
-        assert_chain(fast, {s: r[0] for s, r in ref.items()}, probes, key)
-        sv = m[f"{key}_{FAST}_state"]
-        assert (f32(sv[0]), int(sv[1])) == ref[0][1], key
-        assert_fast_path(fast, exact, key)
-        wf, we = _load_wrapper_chain(m, f"w_{key}_{FAST}"), _load_wrapper_chain(m, f"w_{key}_{EXACT}")
-        _assert_wrapper(wf, wref, wprobes, ("wrapper", key))
-        _assert_wrapper_fast_path(wf, we, ("wrapper", key))
+    fast, exact = _load_chain(m, f"{FAST}"), _load_chain(m, f"{EXACT}")
+    assert_chain(fast, {s: r[0] for s, r in ref.items()}, probes, "caller layout")
+    sv = m[f"{FAST}_state"]
+    assert (f32(sv[0]), int(sv[1])) == ref[0][1]
+    assert_fast_path(fast, exact, "caller layout")
+    wf, we = _load_wrapper_chain(m, f"w_{FAST}"), _load_wrapper_chain(m, f"w_{EXACT}")
+    _assert_wrapper(wf, wref, wprobes, "wrapper")
+    _assert_wrapper_fast_path(wf, we, "wrapper")
 
 
-# ---------------------------------------------------------------- 3. non-interpolating kernel, direct input
+# ---------------------------------------------------------------- 3. non-interpolating kernel, chunked stereo calls
 @pytest.mark.parametrize("flags,lowpass", [(0, 1.0), (espb.BLACKMAN_HARRIS, 1.0), (espb.INCLUDE_LOWPASS, 0.7),
                                            (espb.BLACKMAN_HARRIS | espb.INCLUDE_LOWPASS, 0.7)])
 def test_non_interpolating_kernel(oracle, flags, lowpass):
@@ -500,15 +493,14 @@ def test_non_interpolating_kernel(oracle, flags, lowpass):
 
 
 @pytest.mark.parametrize("taps", [64, 256])
-def test_direct_input(oracle, monkeypatch, taps):
-    """ESPB_DIRECT=1: interleaved stereo read by the kernel through a TMA tensor map; chunked calls of changing size
-    (some shorter than T, which take the staged path and hand the history over), capacity-limited calls."""
-    monkeypatch.setenv("ESPB_DIRECT", "1")
+def test_direct_input(oracle, taps):
+    """Interleaved stereo in chunked calls of changing size (some shorter than T: the carried frames come from more
+    than one earlier call), capacity-limited calls."""
     ns, ch = 70, 2
     geo = (taps, 64, 1.0, 3)
     calls = [(1000, 2000), (10, 50), (900, 300), (64, 500), (2, 9), (1500, 4000), (700, 4000)]
     x = sigs(ns, sum(c[0] for c in calls), ch, seed=1000)
-    check_modes(oracle, ns, ch, geo, x, calls, [R48] * len(calls), ("direct", taps))
+    check_modes(oracle, ns, ch, geo, x, calls, [R48] * len(calls), ("chunked", taps))
 
 
 # ---------------------------------------------------------------- 4. few-series kernel
@@ -887,29 +879,26 @@ def _assert_dyadic(oracle, ns, ch, geo, x, calls, ratios, probes, what, adv=None
     assert any(np.count_nonzero(y) for y, _, _ in runs[FAST][0]), what
 
 
-def test_dyadic_standard_kernel(oracle, monkeypatch):
-    """Dyadic input (samples 0, -0, +-2^k, k in [-14, 0]) on the default standard kernel and on ESPB_BPP=8,
-    ESPB_CHUNK_ROWS=16: fast == exact == plain oracle, bit for bit, with no fused oracle involved."""
+def test_dyadic_standard_kernel(oracle):
+    """Dyadic input (samples 0, -0, +-2^k, k in [-14, 0]) on the standard kernel at T = 256 and at T = 1024 (44.1 ->
+    96 kHz): fast == exact == plain oracle, bit for bit, with no fused oracle involved."""
     ns, ch = 70, 2
     calls = split3(3000, R48)
     x = _dyadic_batch(ns, 3000, ch, seed=0)
     _assert_dyadic(oracle, ns, ch, (256, 256, 1.0, 3), x, calls, [R48] * 3, probes_of(ns), "default")
-    monkeypatch.setenv("ESPB_BPP", "8")
-    monkeypatch.setenv("ESPB_CHUNK_ROWS", "16")
     _assert_dyadic(oracle, ns, ch, (1024, 256, 0.45, 3), x, calls, [f32(44100) / f32(96000)] * 3, probes_of(ns),
-                   "bpp 8 rows 16")
+                   "T 1024")
 
 
-def test_dyadic_non_interpolating_and_direct(oracle, monkeypatch):
-    """Dyadic input on the non-interpolating kernel (flags 2, nearest phase up to F) and on direct input
-    (ESPB_DIRECT=1, stereo)."""
+def test_dyadic_non_interpolating_and_direct(oracle):
+    """Dyadic input on the non-interpolating kernel (flags 2, nearest phase up to F) and on interleaved stereo in
+    chunked calls of changing size (some shorter than T)."""
     ns, ch = 70, 2
     x = _dyadic_batch(ns, 3000, ch, seed=100)
     ratio = f32(44100) / f32(48000)
     _assert_dyadic(oracle, ns, ch, (128, 37, 1.0, 2), x, split3(3000, ratio), [ratio] * 3, probes_of(ns), "ni")
-    monkeypatch.setenv("ESPB_DIRECT", "1")
     calls = [(1000, 2000), (10, 50), (900, 300), (64, 500), (1000, 4000)]
-    _assert_dyadic(oracle, ns, ch, (64, 64, 1.0, 3), x, calls, [R48] * len(calls), probes_of(ns), "direct")
+    _assert_dyadic(oracle, ns, ch, (64, 64, 1.0, 3), x, calls, [R48] * len(calls), probes_of(ns), "chunked")
 
 
 @pytest.mark.parametrize("ns,ch", [(1, 2), (4, 8)])  # 2 and 8 series per lane

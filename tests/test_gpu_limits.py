@@ -8,7 +8,6 @@ Switch                 read                         covered by
 ESPB_GRID_Y_MAX        per process (static)         test_sliced_launches (child process, = 3 and = 1)
 ESPB_GROUPS_FUSED      per context                  test_sliced_launches, test_real_size_clock_groups
 ESPB_FUSE_POST_GROUPS  per call                     test_sliced_launches (mono wrapper: fused post-filter quantiser)
-ESPB_DIRECT            per context (resampleInit)   test_sliced_launches
 ESPB_PPC               per call                     test_sliced_launches
 
 Part a runs every sliced launcher at ordinary sizes with the limit lowered to 3 and to 1 in a child process; each
@@ -170,7 +169,6 @@ RESAMPLE_CASES = [
     ("planes", 1, 40, 3, _planes, {}, {}, "e"),
     ("host", 2, 20, 3, _host, {}, {}, "e"),
     ("flags0", 2, 20, 0, _interleaved, {}, {}, "e"),          # the non-interpolating kernel
-    ("direct", 2, 20, 3, _interleaved, {"ESPB_DIRECT": "1"}, {}, "e"),
     ("ppc1", 2, 20, 3, _interleaved, {"ESPB_PPC": "1"}, {}, "e"),
 ]
 # wrapper: (name, streams, channels, src rate, dst rate, bits, filter position, env)
@@ -347,7 +345,7 @@ def test_sliced_launches(oracle, tmp_path, default_limit_run, limit):
     """ESPB_GRID_Y_MAX = 3 and 1 (read once per process, in a child): every sliced launcher at ordinary sizes, each
     split at least twice — float interleaved 1/2/3/4/6/8 channels, planar, a general stride (frames of channels + 1
     floats, unaligned output rows), few-series and standard kernels, staging overlap on and off, kernel timing on,
-    pointer tables, the host-buffer path, the non-interpolating kernel, direct input, ESPB_PPC=1, the wrapper (int16
+    pointer tables, the host-buffer path, the non-interpolating kernel, ESPB_PPC=1, the wrapper (int16
     and int24, pre- and post-filter, the fused mono post-filter quantiser), the stand-alone biquad in 32-row time
     blocks, a fused set of 7 clock groups and the *_rows quantisers over 10 rows.  The bytes must equal the default
     limit's run in this process, and the oracle (fast mode: its FMA chain) on every series."""

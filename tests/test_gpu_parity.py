@@ -586,11 +586,9 @@ def test_ratio_groups_drifting_ratios_chunked(oracle, mode):
 
 
 @pytest.mark.parametrize("mode", ["exact", "fast"])
-def test_direct_input_path_stereo(oracle, mode, monkeypatch):
-    """ESPB_DIRECT=1: interleaved stereo float input read by the kernel through a TMA tensor map (no staging pass),
-    carried frames from the time-major history.  Chunked calls with changing sizes (some below numTaps, which fall
-    back to the staged path and must hand the history over correctly), capacity-limited calls, a group tail."""
-    monkeypatch.setenv("ESPB_DIRECT", "1")
+def test_direct_input_path_stereo(oracle, mode):
+    """Interleaved stereo float input in chunked calls of changing size (some below numTaps: the carried frames come
+    from more than one earlier call), capacity-limited calls, an empty call, a partial last series group."""
     ch, taps, filters = 2, 64, 64
     ns = 70  # one full group of 64 streams and a partial one
     ratio = f32(48000) / f32(44100)

@@ -3,23 +3,22 @@ default: bit-exact against the oracle in exact mode (frame counts, state, bytes,
 mode, and byte-identical to the default path in both modes wherever the two must agree.
 
 Switch                 read                         covered by
-ESPB_BPP               per context (resampleInit)   test_geometry_matrix, test_chunk_table_limit_per_geometry
-ESPB_CHUNK_ROWS        per context (resampleInit)   test_geometry_matrix, test_chunk_table_limit_per_geometry
 ESPB_G_MBYTES          per context (resampleInit)   test_g_time_slabs*
-ESPB_DIRECT            per context (resampleInit)   test_g_time_slabs_paths
 ESPB_NI                per context (resampleInit)   test_g_time_slabs_paths (on, its default)
-ESPB_SCHED             per context (resampleInit)   test_sequential_schedule*
 ESPB_FS_SLICE_KB       per context (resampleInit)   test_few_series_kernel_switch
 ESPB_STAGE_CTAS        per context (resampleInit)   test_staging_grid_size
 ESPB_OVERLAP           per context (resampleInit)   test_staging_grid_size, test_g_time_slabs
 ESPB_BIQUAD_ONEPASS    per context (biquad_init)    test_standalone_biquad
-ESPB_PPC               per call                     test_passes_per_cta, test_chunk_table_limit_per_geometry
+ESPB_PPC               per call                     test_passes_per_cta, test_chunk_table_limit
 ESPB_HOST_SLABS        per call                     test_host_pipeline_slabs
 ESPB_FS_STAGES         per process (static)         test_few_series_ring_depth (child process)
 ESPB_PCM_CTAS          per process (static)         test_grid_stride_loops (child process)
 ESPB_Q15_CTAS          per process (static)         test_grid_stride_loops (child process)
 ESPB_EXPAND_CTAS       per process (static)         test_grid_stride_loops (child process)
-ESPB_DEBUG             per process                  test_geometry_matrix (names every instantiation it launches)
+ESPB_DEBUG             per process                  test_instantiation_matrix (names every instantiation it launches)
+
+The resampler kernel has one geometry (4 warps per CTA, 32-row chunks, a 2-stage ring) and four instantiations:
+exact / fast x caller-layout / time-major output.
 
 Switches that are cached in a static, and the instantiation report of ESPB_DEBUG (printed once per process), are
 exercised in a child process that writes its results under tmp_path; the parent compares them with the oracle."""
@@ -43,9 +42,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 MODES = (espb.MODE_EXACT, espb.MODE_FAST)
 R48 = f32(48000) / f32(44100)
-# (ESPB_BPP, ESPB_CHUNK_ROWS) -> pipeline stages of that instantiation (resample_kernel.cu:launch_resample)
-GEOMETRIES = {(4, 32): 2, (8, 32): 3, (4, 16): 4, (8, 16): 6, (4, 24): 3, (4, 36): 2}
-TABLE = {(4, 32): 320, (8, 32): 768, (4, 16): 320, (8, 16): 768, (4, 24): 120, (4, 36): 120}  # max_chunks_per_cta
+TABLE = 320  # chunk-table entries a CTA caches (common.hpp: kMaxChunksPerCta)
 # three chained calls: long (> 4096 frames: the staging-overlap path), capacity-limited, uneven
 CALLS = [(4500, 5000), (900, 300), (1202, 1400)]
 
@@ -194,7 +191,7 @@ def _le16(b):
     return np.ascontiguousarray(b).view(np.int16).astype(np.int64)
 
 
-# ---------------------------------------------------------------- 1. resampler geometry matrix
+# ---------------------------------------------------------------- 1. resampler instantiation matrix
 # (ch, streams, taps, flags, forms): 140 series = one full 128-series group and a partial one
 MATRIX = [(2, 70, 256, 3, ("stereo", "planar", "scalar")), (4, 35, 256, 3, ("frame4",)),
           (2, 70, 256, 0, ("stereo",)), (2, 70, 1024, 3, ("stereo",))]
@@ -202,12 +199,9 @@ WRAP_SR, WRAP_DR, WRAP_CALLS = 44100, 48000, [(4500, 4950), (900, 300), (1202, 1
 
 
 def _matrix_cases():
-    for bpp, rows in GEOMETRIES:
-        for ch, ns, taps, flags, forms in MATRIX:
-            if taps == 1024 and (bpp, rows) not in ((4, 32), (4, 24), (4, 36)):
-                continue  # T=1024: the most rows per pass against the 120-entry table of the 24- and 36-row variants
-            for form in forms:
-                yield bpp, rows, ch, ns, taps, flags, form
+    for ch, ns, taps, flags, forms in MATRIX:
+        for form in forms:
+            yield ch, ns, taps, flags, form
 
 
 def _probes(ns, ch):
@@ -215,66 +209,62 @@ def _probes(ns, ch):
 
 
 def _child_geometry_matrix(out_dir):
-    """Every geometry x mode x output form (and the wrapper's time-major output); saves digests + probe rows."""
+    """Every mode x output form (and the wrapper's time-major output); saves digests + probe rows."""
     espb.set_device(0)
     saved = {}
-    for bpp, rows, ch, ns, taps, flags, form in _matrix_cases():
-        _set_env({"ESPB_BPP": bpp, "ESPB_CHUNK_ROWS": rows})
+    for ch, ns, taps, flags, form in _matrix_cases():
         x = signal(ns, sum(c[0] for c in CALLS), ch, seed=1000 + ch)
         for mode in MODES:
             b = espb.ResampleBatch(ns, ch, taps, 256, 1.0, flags, mode=mode)
             b.advance(taps / 2)
             got = device_chain(b, x, CALLS, [R48] * 3, form)
-            key = f"{bpp}_{rows}_{ch}_{taps}_{flags}_{form}_{mode}"
+            key = f"{ch}_{taps}_{flags}_{form}_{mode}"
             saved[key + "_counts"] = np.array([[u, g] for _, u, g in got] + [[int(b.state()[1]), 0]], np.int64)
             saved[key + "_offset"] = np.array([b.state()[0]], f32)
             for k, (y, _, _) in enumerate(got):
                 saved[f"{key}_{k}_sha"] = np.frombuffer(hashlib.sha256(y.tobytes()).digest(), np.uint8)
                 saved[f"{key}_{k}_probes"] = y[_probes(ns, ch)]
             b.free()
-    for bpp, rows in GEOMETRIES:
-        _set_env({"ESPB_BPP": bpp, "ESPB_CHUNK_ROWS": rows})
-        raw = pcm16(70, sum(c[0] for c in WRAP_CALLS), 2, seed=77)
-        for mode in MODES:
-            r = espb.Resampler(70, 4500 * 2, 4950 * 2, WRAP_SR, WRAP_DR, 16, 16, 2, True, True, 256, 256, mode=mode)
-            assert r.policy()["filter"] == "post"
-            got = wrapper_chain(r, raw, 2, WRAP_CALLS, gain_db=2.0)
-            for k, (y, u, g, clips) in enumerate(got):
-                key = f"w_{bpp}_{rows}_{mode}_{k}"
-                saved[key + "_y"] = y
-                saved[key + "_res"] = np.concatenate([[u, g], clips]).astype(np.int64)
-            r.free()
+    raw = pcm16(70, sum(c[0] for c in WRAP_CALLS), 2, seed=77)
+    for mode in MODES:
+        r = espb.Resampler(70, 4500 * 2, 4950 * 2, WRAP_SR, WRAP_DR, 16, 16, 2, True, True, 256, 256, mode=mode)
+        assert r.policy()["filter"] == "post"
+        got = wrapper_chain(r, raw, 2, WRAP_CALLS, gain_db=2.0)
+        for k, (y, u, g, clips) in enumerate(got):
+            key = f"w_{mode}_{k}"
+            saved[key + "_y"] = y
+            saved[key + "_res"] = np.concatenate([[u, g], clips]).astype(np.int64)
+        r.free()
     np.savez(os.path.join(out_dir, "matrix.npz"), **saved)
 
 
-def test_geometry_matrix(oracle, tmp_path):
-    """All six (ESPB_BPP, ESPB_CHUNK_ROWS) geometries, exact and fast, over three chained calls (long / capacity-limited
-    / uneven) of 70 stereo streams, through the interleaved-stereo, planar, 4-channel and scalar (unaligned row) output
-    forms and the wrapper's post-filter path (TMCAP), plus T=1024 and flags=0 (no interpolation: the interpolating
-    kernel with an idle filter, except at (4,32) where the dedicated kernel runs).  Run in a child with ESPB_DEBUG=1:
-    its report must name all 24 resample<BPP,NST,CJ,EXACT,TMCAP> instantiations."""
+def test_instantiation_matrix(oracle, tmp_path):
+    """Exact and fast, over three chained calls (long / capacity-limited / uneven) of 70 stereo streams, through the
+    interleaved-stereo, planar, 4-channel and scalar (unaligned row) output forms and the wrapper's post-filter path
+    (TMCAP), plus T=1024 and flags=0 (no interpolation: the dedicated kernel).  Run in a child with ESPB_DEBUG=1: its
+    report must name exactly the four resample<EXACT,TMCAP> instantiations."""
     err = run_child(tmp_path, "_child_geometry_matrix", {"ESPB_DEBUG": "1"})
-    seen = set(re.findall(r"\[espb\] resample<(\d+),(\d+),(\d+),(\d),(\d)>", err))
-    want = {(str(b), str(n), str(r), str(e), str(t)) for (b, r), n in GEOMETRIES.items() for e in (0, 1) for t in (0, 1)}
-    assert seen == want, sorted(want - seen)
+    seen = set(re.findall(r"\[espb\] resample<([\d,]+)>", err))
+    want = {f"{e},{t}" for e in (0, 1) for t in (0, 1)}
+    assert seen == want, (sorted(want - seen), sorted(seen - want))
     m = np.load(tmp_path / "matrix.npz")
     refs = {}
     for ch, ns, taps, flags, _ in MATRIX:
         x = signal(ns, sum(c[0] for c in CALLS), ch, seed=1000 + ch)
         refs[(ch, taps, flags)] = {s: oracle_chain(oracle, x[s], ch, taps, 256, 1.0, flags, CALLS, [R48] * 3)
                                    for s in _probes(ns, ch)}
-    for bpp, rows, ch, ns, taps, flags, form in _matrix_cases():
+    for ch, ns, taps, flags, form in _matrix_cases():
         ref = refs[(ch, taps, flags)]
         probes = _probes(ns, ch)
         for mode in MODES:
-            key = f"{bpp}_{rows}_{ch}_{taps}_{flags}_{form}_{mode}"
-            base = f"4_32_{ch}_{taps}_{flags}_stereo_{mode}" if form != "frame4" else f"4_32_{ch}_{taps}_{flags}_frame4_{mode}"
+            key = f"{ch}_{taps}_{flags}_{form}_{mode}"
+            base = f"{ch}_{taps}_{flags}_stereo_{mode}" if form != "frame4" else key
             counts = m[key + "_counts"]
             ochain, ostate = ref[probes[0]]
             assert [tuple(c) for c in counts[:3]] == [(u, g) for _, u, g in ochain], key
             assert (m[key + "_offset"][0], int(counts[3][0])) == ostate, key
             for k in range(3):
-                # identical bytes to the default geometry (and, for the other layouts, to its interleaved output)
+                # the other layouts: identical bytes to the interleaved output
                 assert bits_equal(m[f"{key}_{k}_sha"], m[f"{base}_{k}_sha"]), (key, k)
                 for i, s in enumerate(probes):
                     yo = ref[s][0][k][0]
@@ -287,53 +277,48 @@ def test_geometry_matrix(oracle, tmp_path):
     wref = {s: oracle_wrapper_chain(oracle, raw[s], 2, WRAP_SR, WRAP_DR, WRAP_CALLS, gain_db=2.0)
             for s in (0, 31, 32, 69)}
     clipped = 0
-    for bpp, rows in GEOMETRIES:
-        for mode in MODES:
-            for k in range(3):
-                key, base = f"w_{bpp}_{rows}_{mode}_{k}", f"w_4_32_{mode}_{k}"
-                y, res = m[key + "_y"], m[key + "_res"]
-                assert bits_equal(y, m[base + "_y"]) and np.array_equal(res, m[base + "_res"]), key
-                for s, chain in wref.items():
-                    yo, uo, go, co = chain[k]
-                    assert (int(res[0]), int(res[1])) == (uo, go), (key, s)
-                    if mode == espb.MODE_EXACT:
-                        assert bits_equal(y[s], yo) and int(res[2 + s]) == co, (key, s)
-                        clipped += co
-                    else:  # fast mode: within one LSB of the 16-bit output
-                        assert np.max(np.abs(_le16(y[s]) - _le16(yo))) <= 1, (key, s)
+    for mode in MODES:
+        for k in range(3):
+            key = f"w_{mode}_{k}"
+            y, res = m[key + "_y"], m[key + "_res"]
+            for s, chain in wref.items():
+                yo, uo, go, co = chain[k]
+                assert (int(res[0]), int(res[1])) == (uo, go), (key, s)
+                if mode == espb.MODE_EXACT:
+                    assert bits_equal(y[s], yo) and int(res[2 + s]) == co, (key, s)
+                    clipped += co
+                else:  # fast mode: within one LSB of the 16-bit output
+                    assert np.max(np.abs(_le16(y[s]) - _le16(yo))) <= 1, (key, s)
     assert clipped > 0  # the +2 dB gain clips: the clip counts were compared
 
 
-# ---------------------------------------------------------------- 2. chunk-table limit per geometry
-def _max_chunks(taps, state, n_in, n_out, ratio, bpp, rows):
-    _, _, pcb = espb.plan_passes(taps, 256, 3, float(state[0]), state[1], n_in, n_out, ratio, bpp, rows, False)
+# ---------------------------------------------------------------- 2. chunk-table limit
+def _max_chunks(taps, state, n_in, n_out, ratio):
+    # the kernel's plan: passes of 4 blocks, 32-row chunks
+    _, _, pcb = espb.plan_passes(taps, 256, 3, float(state[0]), state[1], n_in, n_out, ratio, 4, 32)
     return int(np.max(np.diff(pcb)))
 
 
-def _threshold(taps, state, n_in, n_out, bpp, rows):
-    """(accepted, refused) float32 ratios either side of the table limit of this geometry, for this call's plan."""
-    limit = TABLE[(bpp, rows)]
+def _threshold(taps, state, n_in, n_out):
+    """(accepted, refused) float32 ratios either side of the table limit, for this call's plan."""
+    limit = TABLE
     lo, hi = f32(0.0005), f32(0.05)
-    assert _max_chunks(taps, state, n_in, n_out, lo, bpp, rows) > limit >= _max_chunks(taps, state, n_in, n_out, hi,
-                                                                                        bpp, rows)
+    assert _max_chunks(taps, state, n_in, n_out, lo) > limit >= _max_chunks(taps, state, n_in, n_out, hi)
     for _ in range(60):
         mid = f32((float(lo) + float(hi)) / 2)
         if mid in (lo, hi):
             break
-        if _max_chunks(taps, state, n_in, n_out, mid, bpp, rows) > limit:
+        if _max_chunks(taps, state, n_in, n_out, mid) > limit:
             lo = mid
         else:
             hi = mid
     return hi, lo
 
 
-@pytest.mark.parametrize("bpp,rows", list(GEOMETRIES))
-def test_chunk_table_limit_per_geometry(oracle, monkeypatch, bpp, rows):
-    """Per geometry, the ratio where one pass's chunks first exceed the CTA's chunk table (320 / 768 / 120 entries):
-    just above it the call is refused (ESPB_ERR_ARG) before anything runs and the context stays usable; just below
-    it the call runs and is bit-exact.  ESPB_PPC=64 at the accepted ratio exercises the clamp ppc * chunks <= table."""
-    monkeypatch.setenv("ESPB_BPP", str(bpp))
-    monkeypatch.setenv("ESPB_CHUNK_ROWS", str(rows))
+def test_chunk_table_limit(oracle, monkeypatch):
+    """The ratio where one pass's chunks first exceed the CTA's chunk table (320 entries): just above it the call is
+    refused (ESPB_ERR_ARG) before anything runs and the context stays usable; just below it the call runs and is
+    bit-exact.  ESPB_PPC=64 at the accepted ratio exercises the clamp ppc * chunks <= table."""
     L = espb.lib()
     ns, ch, taps, n_in = 70, 2, 256, 60000
     n_out = 4000
@@ -341,7 +326,7 @@ def test_chunk_table_limit_per_geometry(oracle, monkeypatch, bpp, rows):
     probe = ns - 1
     b = espb.ResampleBatch(ns, ch, taps, 256, 1.0, 3, mode=espb.MODE_EXACT)
     b.advance(taps / 2)
-    ok, bad = _threshold(taps, b.state(), n_in, n_out, bpp, rows)
+    ok, bad = _threshold(taps, b.state(), n_in, n_out)
     assert float(ok) / float(bad) < 1.001
     d_in = espb.DeviceBuffer.from_numpy(x)
     d_out = espb.DeviceBuffer(ns * n_out * ch * 4)
@@ -415,9 +400,8 @@ def test_g_time_slabs(oracle, monkeypatch, mode):
 
 def test_g_time_slabs_paths(oracle, monkeypatch):
     """G slabs on the other kernels and entry points, each against the same configuration with the default budget
-    and against the oracle: the non-interpolating kernel (half-size G rows), direct input (ESPB_DIRECT=1, split pass
-    plan), the host-buffer pipeline (stream slabs serial on one CUDA stream, G re-expanded per slab) and the wrapper
-    (device and host path)."""
+    and against the oracle: the non-interpolating kernel (half-size G rows), the host-buffer pipeline (stream slabs
+    serial on one CUDA stream, G re-expanded per slab) and the wrapper (device and host path)."""
     ns, ch, taps = 70, 2, 256
     total = sum(c[0] for c in CALLS)
     x = signal(ns, total, ch, seed=3100)
@@ -432,16 +416,17 @@ def test_g_time_slabs_paths(oracle, monkeypatch):
             monkeypatch.delenv(k)
         return b
 
-    for flags, env in ((espb.BLACKMAN_HARRIS, {}), (3, {"ESPB_DIRECT": "1"})):
-        ref = {s: oracle_chain(oracle, x[s], ch, taps, 256, 1.0, flags, CALLS, [R48] * 3)[0] for s in probes}
-        for mode in MODES:
-            base = device_chain(batch(flags, env, mode), x, CALLS, [R48] * 3)
-            b = batch(flags, dict(env, ESPB_G_MBYTES="1"), mode)
-            (y, u, g), launches = _resample_launches(b, x[:, : CALLS[0][0] * ch], *CALLS[0], R48)
-            assert launches > 1
-            got = [(y, u, g)] + device_chain(b, x[:, u * ch:], CALLS[1:], [R48] * 2)
-            same_chain(got, base, (flags, env, mode))
-            check_against_oracle(got, ref, probes, mode, (flags, env))
+    # the non-interpolating kernel
+    flags = espb.BLACKMAN_HARRIS
+    ref = {s: oracle_chain(oracle, x[s], ch, taps, 256, 1.0, flags, CALLS, [R48] * 3)[0] for s in probes}
+    for mode in MODES:
+        base = device_chain(batch(flags, {}, mode), x, CALLS, [R48] * 3)
+        b = batch(flags, {"ESPB_G_MBYTES": "1"}, mode)
+        (y, u, g), launches = _resample_launches(b, x[:, : CALLS[0][0] * ch], *CALLS[0], R48)
+        assert launches > 1
+        got = [(y, u, g)] + device_chain(b, x[:, u * ch:], CALLS[1:], [R48] * 2)
+        same_chain(got, base, ("ni", mode))
+        check_against_oracle(got, ref, probes, mode, "ni")
     # host-buffer pipeline: every stream slab re-expands its G slabs on the one CUDA stream
     ref = {s: oracle_chain(oracle, x[s], ch, taps, 256, 1.0, 3, CALLS, [R48] * 3)[0] for s in probes}
     for mode in MODES:
@@ -571,29 +556,21 @@ VS_ORACLE = [  # the geometries of test_gpu_parity.py::test_resampler_vs_oracle
 
 
 @pytest.mark.parametrize("case", VS_ORACLE)
-def test_sequential_schedule(oracle, monkeypatch, case):
-    """ESPB_SCHED=seq: the per-output schedule built on the host and finished by espb_finalize_kernel instead of the
-    closed form expanded on the device.  Two chained calls; bytes, counts and state equal the closed form's and the
-    oracle's."""
+def test_sequential_schedule(oracle, case):
+    """The schedule the device expands from its closed form, over two chained calls: bytes, counts and end state equal
+    those of the oracle's sequential state machine (the second call starts from the state the first one left)."""
     ch, ns, taps, filters, lp, flags, ratio, n_in = case
     calls = [(n_in // 3 + 1, int((n_in // 3 + 1) * float(ratio)) + 40), (n_in - n_in // 3 - 1, int(n_in * float(ratio)))]
     x = signal(ns, n_in, ch, seed=6000 + ns)
     probes = sorted({0, ns - 1})
     ref = {s: oracle_chain(oracle, x[s], ch, taps, filters, lp, flags, calls, [ratio] * 2) for s in probes}
     for mode in MODES:
-        runs = {}
-        for sched in ("seq", None):
-            if sched:
-                monkeypatch.setenv("ESPB_SCHED", sched)
-            else:
-                monkeypatch.delenv("ESPB_SCHED", raising=False)
-            b = espb.ResampleBatch(ns, ch, taps, filters, lp, flags, mode=mode)
-            b.advance(taps / 2)
-            runs[sched] = (device_chain(b, x, calls, [ratio] * 2, "scalar" if ch % 2 else "stereo"), b.state())
-            b.free()
-        same_chain(runs["seq"][0], runs[None][0], ("seq", mode))
-        assert runs["seq"][1] == runs[None][1] == ref[0][1]
-        check_against_oracle(runs["seq"][0], {s: r[0] for s, r in ref.items()}, probes, mode, "seq")
+        b = espb.ResampleBatch(ns, ch, taps, filters, lp, flags, mode=mode)
+        b.advance(taps / 2)
+        got = device_chain(b, x, calls, [ratio] * 2, "scalar" if ch % 2 else "stereo")
+        assert b.state() == ref[0][1]
+        b.free()
+        check_against_oracle(got, {s: r[0] for s, r in ref.items()}, probes, mode, "closed form")
 
 
 # ---------------------------------------------------------------- 7. few-series <-> standard kernel in one context

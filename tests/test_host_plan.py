@@ -29,7 +29,7 @@ def test_library_loads_and_exports_every_declared_symbol():
     assert len(names) >= 50
     missing = [n for n in names if not hasattr(L, n)]
     assert not missing, missing
-    assert L.espb_abi_version() == 1
+    assert L.espb_abi_version() == 2
     assert os.path.basename(espb.library_path()) == "libesp_audio_b200.so"
 
 
@@ -211,21 +211,21 @@ def test_cpp_shim_compiles_and_links(tmp_path):
     subprocess.run(["gcc", "-std=c99", "-fsyntax-only", "-I", os.path.join(root, "include"), str(csrc)], check=True)
 
 
-@pytest.mark.parametrize("taps,ratio,n_in,split", [(256, 48000 / 44100, 5000, False), (256, 48000 / 44100, 5000, True),
-                                                  (64, 0.37, 3001, True), (1024, 44100 / 96000, 9000, True),
-                                                  (32, 3.0, 700, True), (8, 1.0, 100, True),
-                                                  # the call lengths of test_gpu_limits.py's real-size tests
-                                                  (32, 48000 / 44100, 2_100_000, False),
-                                                  (32, 48000 / 44100, 4_200_000, True)])
-def test_pass_plan_covers_every_window(taps, ratio, n_in, split):
+@pytest.mark.parametrize("taps,ratio,n_in,bpp", [(256, 48000 / 44100, 5000, 4), (64, 0.37, 3001, 4),
+                                                (1024, 44100 / 96000, 9000, 4), (32, 3.0, 700, 4), (8, 1.0, 100, 4),
+                                                # the non-interpolating kernel's plan: 8 blocks per pass
+                                                (256, 44100 / 48000, 5000, 8),
+                                                # the call lengths of test_gpu_limits.py's real-size tests
+                                                (32, 48000 / 44100, 2_100_000, 4),
+                                                (32, 48000 / 44100, 4_200_000, 4)])
+def test_pass_plan_covers_every_window(taps, ratio, n_in, bpp):
     """The chunk table the kernel sweeps (host logic, no GPU): every output's window lies inside the chunks of its
-    pass, chunks of a pass are contiguous in time, and the split form the direct-input kernel needs never straddles
-    input frame 0, starts history chunks on multiples of 4 rows and input chunks on even frames."""
+    pass, and the chunks of a pass are contiguous in time."""
     f32 = np.float32
-    filters, flags, bpp, rows = 64, 3, 4, 32
+    filters, flags, rows = 64, 3, 32
     n_out = int(n_in * ratio) + 16
     sched = espb.plan_schedule(taps, filters, flags, float(taps // 2), taps, n_in, n_out, f32(ratio))
-    cs, cp, pcb = espb.plan_passes(taps, filters, flags, float(taps // 2), taps, n_in, n_out, f32(ratio), bpp, rows, split)
+    cs, cp, pcb = espb.plan_passes(taps, filters, flags, float(taps // 2), taps, n_in, n_out, f32(ratio), bpp, rows)
     gen = sched["generated"]
     assert gen > 0 and len(pcb) == (gen + bpp * 8 - 1) // (bpp * 8) + 1 and pcb[0] == 0 and pcb[-1] == len(cs)
     ws = sched["ws"]
@@ -235,19 +235,9 @@ def test_pass_plan_covers_every_window(taps, ratio, n_in, split):
         starts = cs[a:b].astype(np.int64)
         lo, hi = int(ws[p * bpp * 8]), int(ws[min((p + 1) * bpp * 8, gen) - 1]) + taps
         covered = np.zeros(hi - lo, bool)
-        for k, j in enumerate(starts):
-            end = j + rows
-            if split and j < 0:
-                assert j % 4 == 0
-                end = min(end, 0)  # rows from frame 0 on belong to the chunk that starts there
-                if hi > 0 >= lo:
-                    pass
-            elif split:
-                assert j % 2 == 0 and j >= 0
-            if k + 1 < len(starts):
-                nxt = starts[k + 1]
-                assert nxt == j + rows or (split and j < 0 <= j + rows and nxt == 0) or (split and j < 0 and nxt == 0)
-            covered[max(j, lo) - lo: max(min(end, hi), lo) - lo] = True
+        assert starts[0] == lo and np.all(np.diff(starts) == rows)
+        for j in starts:
+            covered[max(j, lo) - lo: max(min(j + rows, hi), lo) - lo] = True
         assert covered.all(), (p, lo, hi, starts)
 
 

@@ -7,7 +7,7 @@ here=$(cd "$(dirname "$0")/.." && pwd)
 src=$here/esp-audio-libs_b200/csrc
 out=$here/esp-audio-libs_b200/variants
 mkdir -p $out/build_$name
-for f in api.cu resample_kernel.cu resample_direct_kernel.cu resample_ni_kernel.cu resample_fs_kernel.cu pcm_kernels.cu biquad_kernel.cu util_kernels.cu q15_kernels.cu groups.cu multi.cu plan.cpp wav.cpp; do
+for f in api.cu resample_kernel.cu resample_ni_kernel.cu resample_fs_kernel.cu pcm_kernels.cu biquad_kernel.cu util_kernels.cu q15_kernels.cu groups.cu multi.cu plan.cpp wav.cpp; do
   ( nvcc -O3 -std=c++17 -lineinfo -gencode arch=compute_100a,code=sm_100a -Xcompiler -fPIC,-O2,-ffp-contract=off "$@" -c $src/$f -o $out/build_$name/$f.o ) &
 done
 wait

@@ -1,6 +1,6 @@
 #!/bin/bash
 # Resampler-kernel variants on the BASELINE configs[1] workload: prints kernel ms and roofline fraction per setting.
-# usage: tools/sweep_kernel.sh "ESPB_CHUNK_ROWS=16" "ESPB_CHUNK_ROWS=16 ESPB_PPC=10" ...
+# usage: tools/sweep_kernel.sh "ESPB_PPC=0" "ESPB_PPC=10" ...
 mkdir -p gpurun_out
 for cfg in "$@"; do
   env $cfg python bench.py --steps 10 --warmup 3 --no-e2e --no-cpu-baseline 2>/dev/null | python -c "
